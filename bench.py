@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- ForceAtlas iterations/s and pair-interactions/s on B200 (BASELINE.json metric).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR] [--workload ...]
 
 Workload (config.workload): BASELINE config 4, the flat single-level ForceAtlas iteration on a
 500 000-vertex random geometric graph (avg degree 10), all-pairs repulsion, d = 2, FP64 like the
@@ -285,6 +285,11 @@ def run_ours(args):
     launches = ctx.launches - launches0
     ms = sum(a.elapsed_time(b) for a, b in ev)
     clocks = sampler.result()
+    if args.dump_outputs and rank == 0:
+        outputs = {"coords": plan.download()}
+        if world == 1:  # at N > 1 each rank holds the forces of its own rows only
+            outputs["forces"] = plan.download_forces()
+        dump_outputs(args.dump_outputs, outputs)
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
@@ -367,6 +372,24 @@ def run_ours(args):
     if parity["parity_max_err"] > PARITY_TOL or not parity["parity_ok"]:
         log("[bench] PARITY FAILURE: %r" % (parity,))
         sys.exit(3)
+
+
+DUMP_BYTES = 60 << 20  # under 64 MB in all, .npy headers included
+
+
+def dump_outputs(path, arrays):
+    """Writes each n-row array as <path>/<name>.npy (float64).  Above DUMP_BYTES in all, the same
+    fixed, seeded sample of rows is written for every array, with the row indices as rows.npy."""
+    os.makedirs(path, exist_ok=True)
+    n = next(iter(arrays.values())).shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values())
+    if n * row_bytes > DUMP_BYTES:
+        k = DUMP_BYTES // (row_bytes + 8)
+        rows = np.sort(np.random.default_rng(0).choice(n, size=k, replace=False))
+        arrays = dict({name: a[rows] for name, a in arrays.items()}, rows=rows.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), np.ascontiguousarray(a, dtype=np.float64))
+    log("[bench] outputs of the last timed step written to %s: %s" % (path, sorted(arrays)))
 
 
 PARITY_TOL = 1e-10  # FP64 forces, relative to the vertex's conditioning scale (tests/helpers.py)
@@ -775,6 +798,8 @@ def main():
     ap.add_argument("--galerkin-n", type=int, default=1_000_000)
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--no-attraction", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the coordinates (and at N = 1 the forces) of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -6,9 +6,10 @@
 Runs `partition::partition(A, cf, false, true, 1.0, 2, false)` (src/partitioner.cpp:1550-1893, the call
 shape of examples/embedder.cpp:187) through oracle/_ref (the unmodified reference compiled by
 oracle/Makefile) on the synthetic graph the generator in graph-embed_b200/graphs.py produces for the
-given seed, and stores ONLY the vertex->aggregate map of every level (int32) plus the generator's
-arguments and a checksum of the graph: the graph itself is regenerated from the seed wherever the
-fixture is used (tests/helpers.py::ref_hierarchy), and the checksum catches a generator that drifted.
+given seed, and stores ONLY the vertex->aggregate map of every level, relative to that level's graph
+(tests/helpers.py::encode_aggregates), plus the generator's arguments and a checksum of the graph: the
+graph itself is regenerated from the seed wherever the fixture is used
+(tests/helpers.py::load_ref_hierarchy), and the checksum catches a generator that drifted.
 Needs /root/reference (build container only); the partition of R-MAT-20 takes ~20 CPU-minutes, which
 is why the result is committed.
 """
@@ -22,7 +23,9 @@ import numpy as np
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(os.path.dirname(HERE))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.dirname(HERE))
 import __graft_entry__ as entry  # noqa: E402
+from helpers import pack_i32, encode_aggregates  # noqa: E402
 
 entry.load_package()
 O = entry.load_oracle()
@@ -64,6 +67,7 @@ def main():
            "n": np.int64(A.shape[0]), "nnz": np.int64(A.nnz), "digest": graph_digest(A),
            "L": np.int32(len(Ps)), "partition_seconds": np.float64(secs),
            "partition_threads": np.int32(threads)}
+    As = G.hierarchy_from(A, Ps)
     for l, P in enumerate(Ps):
         # P_T has one unit entry per column and members ascending per row (interpolationMatrix,
         # src/partitioner.cpp:29-65): the vertex->aggregate map determines it completely.
@@ -72,12 +76,13 @@ def main():
         rebuilt = G.aggregation_matrix(agg, P.shape[0])
         assert np.array_equal(rebuilt.indptr, P.indptr) and np.array_equal(rebuilt.indices, P.indices), \
             "members not ascending: the map does not determine P_T at level %d" % l
-        out["agg%d" % l] = agg
+        link, root_ids = encode_aggregates(As[l], P)
+        out["link%d" % l], out["roots%d" % l] = pack_i32(link), pack_i32(root_ids)
         s = np.diff(P.indptr).astype(np.int64)
         print("level", l, "n", P.shape[1], "aggregates", P.shape[0], "max", int(s.max()),
               "pairs", int((s * (s - 1)).sum()), flush=True)
     name = "refhier_%s%d.npz" % (kind, arg)
-    np.savez_compressed(os.path.join(HERE, name), **out)
+    np.savez(os.path.join(HERE, name), **out)  # the members are xz-compressed already
     print("wrote", name, os.path.getsize(os.path.join(HERE, name)), "bytes")
 
 

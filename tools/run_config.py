@@ -1,7 +1,7 @@
 """One-off full-size runs of the BASELINE configs through ge_embed (single GPU):
   python tools/run_config.py config3 | config5 [n_points] | config2 | config1  [--ref] [--cpu-ref]
 --ref      use the hierarchy of the REFERENCE's partitioner cached under tests/golden/refhier_*.npz
-           (config3: R-MAT-20; config5: Delaunay of n_points = 1000000 or 4000000) instead of the
+           (config3: R-MAT-20; config5: Delaunay of n_points = 1000000) instead of the
            stand-in generator graphs.coarsen
 --gpus=N   one context over N GPUs of the box (large levels sharded by aggregates)
 --cpu-ref  also time the compiled reference's embed() (oracle/_ref, all host threads) on the same
@@ -44,7 +44,7 @@ def main():
     if use_ref:
         sys.path.insert(0, os.path.join(ROOT, "tests"))
         from helpers import load_ref_hierarchy
-        key = {"config3": "rmat20", "config5": "delaunay%d" % int(arg or 4_000_000)}[name]
+        key = {"config3": "rmat20", "config5": "delaunay%d" % int(arg or 1_000_000)}[name]
         As, Ps, meta = load_ref_hierarchy(graphs, key)
         A, cf, dim = As[0], meta["cf"], 3
         t_gen, t_coarsen = time.time() - t, meta["partition_seconds"]
