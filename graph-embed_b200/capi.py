@@ -74,6 +74,8 @@ SYMBOLS = [
     "ge_flat_symmetric_share", "ge_galerkin", "ge_level_radii_device",
     "ge_context_create_multi", "ge_context_device_count",
     "ge_flat_symmetric_pass_share", "ge_embed_aggregate_ranges", "ge_embed_aggregate_owners",
+    "ge_coarsen_options_default", "ge_coarsen", "ge_hierarchy_levels", "ge_hierarchy_graph",
+    "ge_hierarchy_aggregation", "ge_hierarchy_destroy",
 ]
 
 _lib = None
@@ -98,7 +100,9 @@ def lib():
         L.ge_reference_uniform.argtypes = [C.c_uint32, C.c_int64, _pd]
         L.ge_context_create.argtypes = [C.c_int, C.c_void_p, C.POINTER(C.c_void_p)]
         L.ge_context_bytes.restype = None
-        for name in ("ge_context_destroy", "ge_flat_plan_destroy", "ge_flat_plan_swap"):
+        L.ge_hierarchy_levels.argtypes = [C.c_void_p]
+        L.ge_hierarchy_levels.restype = C.c_int32
+        for name in ("ge_context_destroy", "ge_flat_plan_destroy", "ge_flat_plan_swap", "ge_hierarchy_destroy"):
             getattr(L, name).argtypes = [C.c_void_p]
             getattr(L, name).restype = None
         _lib = L
@@ -125,6 +129,26 @@ def _ptr(a, typ):
 class GalerkinStats(C.Structure):
     _fields_ = [("device_ms", C.c_double), ("total_ms", C.c_double), ("kernel_launches", C.c_int64),
                 ("segments_shared", C.c_int64), ("segments_global", C.c_int64), ("nnz_out", C.c_int64)]
+
+
+class CoarsenOptions(C.Structure):
+    _fields_ = [("coarsening_factor", C.c_double), ("min_coarse", C.c_int32), ("max_levels", C.c_int32),
+                ("seed", C.c_uint32)]
+
+
+class CoarsenStats(C.Structure):
+    _fields_ = [("total_ms", C.c_double), ("device_ms", C.c_double), ("rounds", C.c_int64),
+                ("kernel_launches", C.c_int64)]
+
+
+def _csr_copy(c, with_data=True):
+    """scipy CSR copy of a ge_csr view (int32 / float64)."""
+    import scipy.sparse as sp
+    nnz = int(c.nnz)
+    indptr = np.ctypeslib.as_array(c.indptr, shape=(c.rows + 1,)).copy()
+    indices = np.ctypeslib.as_array(c.indices, shape=(nnz,)).copy() if nnz else np.zeros(0, np.int32)
+    data = np.ctypeslib.as_array(c.data, shape=(nnz,)).copy() if nnz else np.zeros(0)
+    return sp.csr_matrix((data, indices, indptr), shape=(c.rows, c.cols))
 
 
 class CsrView:
@@ -329,6 +353,33 @@ class Context:
         if with_stats:
             return Ac, {f: getattr(st, f) for f, _ in st._fields_}
         return Ac
+
+    def coarsen(self, A, coarsening_factor=0.25, min_coarse=64, max_levels=32, seed=0):
+        """ge_coarsen: the hierarchy built on the device -> (As, P_Ts, stats) as scipy CSR, in the
+        shape graphs.coarsen returns (As[0] is A)."""
+        import scipy.sparse as sp
+        A = sp.csr_matrix(A)
+        a = CsrView(A)
+        opt = CoarsenOptions()
+        lib().ge_coarsen_options_default(C.byref(opt))
+        opt.coarsening_factor, opt.min_coarse = float(coarsening_factor), int(min_coarse)
+        opt.max_levels, opt.seed = int(max_levels), int(seed)
+        st = CoarsenStats()
+        h = C.c_void_p()
+        _check(lib().ge_coarsen(self.h, a.ref(), C.byref(opt), C.byref(h), C.byref(st)))
+        try:
+            L = int(lib().ge_hierarchy_levels(h))
+            As = [sp.csr_matrix((a.data, a.indices, a.indptr), shape=A.shape)]
+            Ps = []
+            for l in range(L):
+                c = Csr()
+                _check(lib().ge_hierarchy_aggregation(h, l, C.byref(c)))
+                Ps.append(_csr_copy(c))
+                _check(lib().ge_hierarchy_graph(h, l + 1, C.byref(c)))
+                As.append(_csr_copy(c))
+        finally:
+            lib().ge_hierarchy_destroy(h)
+        return As, Ps, {f: getattr(st, f) for f, _ in st._fields_}
 
     def flat_plan(self, A, dim, params, rows=None, symmetric=None):
         """rows=(r0, r1): ordered row-block plan; symmetric=(rank, world): that rank's plan of a

@@ -869,6 +869,8 @@ struct ge_flat_plan {
   std::unique_ptr<ge::FlatSolver> solver;
 };
 
+struct ge_hierarchy : ge::HostHierarchy {};
+
 using namespace ge;
 
 extern "C" {
@@ -1188,6 +1190,67 @@ ge_status ge_galerkin(ge_context* ctx, const ge_csr* A, const ge_csr* P_T, int32
     GE_REQUIRE(*nnz_out <= capacity, "output capacity too small (see *nnz_out)");
   });
 }
+
+void ge_coarsen_options_default(ge_coarsen_options* opt) {
+  std::memset(opt, 0, sizeof(*opt));
+  opt->coarsening_factor = 0.25;
+  opt->min_coarse = 64;
+  opt->max_levels = 32;
+  opt->seed = 0;
+}
+
+ge_status ge_coarsen(ge_context* ctx, const ge_csr* A, const ge_coarsen_options* opt,
+                     ge_hierarchy** out, ge_coarsen_stats* stats) {
+  return guarded([&] {
+    GE_REQUIRE(out != nullptr, "out is null");
+    *out = nullptr;
+    int count = 0;
+    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
+      cudaGetLastError();
+      set_error("no usable CUDA device (this library has no CPU fallback)");
+      throw Fail{GE_ERR_NO_DEVICE};
+    }
+    require_ctx(ctx);  // a multi-device context: its first device
+    check_csr(A, "A");
+    GE_REQUIRE(opt != nullptr, "options are null");
+    std::unique_ptr<ge_hierarchy> h(new ge_hierarchy);
+    coarsen(ctx, *A, *opt, *h, stats);
+    *out = h.release();
+  });
+}
+
+int32_t ge_hierarchy_levels(const ge_hierarchy* h) { return h ? (int32_t)h->aggs.size() : 0; }
+
+namespace {
+ge_csr csr_view(const HostHierarchy::Csr& c) {
+  ge_csr v;
+  v.rows = c.rows;
+  v.cols = c.cols;
+  v.nnz = (int64_t)c.indices.size();
+  v.indptr = c.indptr.data();
+  v.indices = c.indices.data();
+  v.data = c.data.data();
+  return v;
+}
+}  // namespace
+
+ge_status ge_hierarchy_graph(const ge_hierarchy* h, int32_t l, ge_csr* out) {
+  return guarded([&] {
+    GE_REQUIRE(h != nullptr && out != nullptr, "null argument");
+    GE_REQUIRE(l >= 1 && l <= (int32_t)h->graphs.size(), "level out of range (1 .. L)");
+    *out = csr_view(h->graphs[l - 1]);
+  });
+}
+
+ge_status ge_hierarchy_aggregation(const ge_hierarchy* h, int32_t l, ge_csr* out) {
+  return guarded([&] {
+    GE_REQUIRE(h != nullptr && out != nullptr, "null argument");
+    GE_REQUIRE(l >= 0 && l < (int32_t)h->aggs.size(), "level out of range (0 .. L-1)");
+    *out = csr_view(h->aggs[l]);
+  });
+}
+
+void ge_hierarchy_destroy(ge_hierarchy* h) { delete h; }
 
 void ge_reference_uniform(uint32_t seed, int64_t count, double* out) {
   reference_uniform(seed, count, out);

@@ -206,6 +206,46 @@ RadiiLevel radii_level_of(const PrefetchedGraph& g, int mc);
 // ---- ge_galerkin.cu ----------------------------------------------------------------------------
 int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P_T, int32_t* c_indptr,
                  int32_t* c_indices, double* c_data, int64_t capacity, ge_galerkin_stats* stats);
+// A graph and its aggregation already on the device (every pointer is a device pointer).
+// Segment a of the product is the entries of the rows of aggregate a's members, in P_T order:
+// segoff [m+1] = first entry of each segment, rowoff [n] = offset of row i inside its segment.
+struct GalerkinInput {
+  int n = 0, m = 0;
+  const int* I = nullptr;
+  const int* J = nullptr;
+  const double* W = nullptr;  // nullptr: unit weights
+  const int* vA = nullptr;    // vertex -> aggregate [n]
+  const int* Pptr = nullptr;  // P_T.indptr [m+1]
+  const int* Pidx = nullptr;  // P_T.indices [n]
+  const int* rowoff = nullptr;
+  const int* segoff = nullptr;
+};
+// The product on the device.  segoff_host: host copy of in.segoff (the size classes of the segments
+// are sorted out on the host).  outptr receives the row pointers [m+1]; when nnz(A_c) <= capacity,
+// outcol / outval receive the columns and values.  c_indptr (host, may be null) receives a copy of
+// the row pointers.  Returns nnz(A_c) (synchronises the stream once); stats: the segment counts and
+// nnz_out only.  start (optional) is recorded after the size classes are uploaded, just before the
+// first kernel.
+int64_t galerkin_device(ge_context* ctx, const GalerkinInput& in, const int* segoff_host,
+                        int32_t* c_indptr, DevBuf<int>& outptr, DevBuf<int>& outcol,
+                        DevBuf<double>& outval, int64_t capacity, ge_galerkin_stats* stats,
+                        cudaEvent_t start = nullptr);
+// Exclusive prefix sum of d_in [n] into d_out [n+1] (d_out[n] = total), on the context stream.
+void exclusive_scan(ge_context* ctx, const int* d_in, int n, int* d_out);
+
+// ---- ge_coarsen.cu ---------------------------------------------------------------------------
+// Builds the hierarchy of ge_coarsen (include/graph_embed_b200.h) on the context's device.
+struct HostHierarchy {
+  struct Csr {
+    int rows = 0, cols = 0;
+    std::vector<int> indptr, indices;
+    std::vector<double> data;
+  };
+  std::vector<Csr> graphs;  // As[1..L]
+  std::vector<Csr> aggs;    // P_T[0..L-1]
+};
+void coarsen(ge_context* ctx, const ge_csr& A, const ge_coarsen_options& opt, HostHierarchy& out,
+             ge_coarsen_stats* stats);
 
 // ---- ge_multi.cu ---------------------------------------------------------------------------------
 void multi_attach(ge_context* ctx, int ndev, const int* devices);

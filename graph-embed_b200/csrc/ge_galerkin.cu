@@ -414,79 +414,26 @@ __global__ void __launch_bounds__(256) k_gal_compact(const int* __restrict__ seg
 
 }  // namespace
 
-// Returns nnz(A_c); fills c_indptr always, c_indices / c_data when capacity suffices.
-int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P, int32_t* c_indptr,
-                 int32_t* c_indices, double* c_data, int64_t capacity, ge_galerkin_stats* stats) {
-  const int n = A.rows, m = P.rows;
-  GE_REQUIRE(A.rows == A.cols, "A must be square");
-  GE_REQUIRE(P.cols == n, "P_T.cols != A.rows");
-  GE_REQUIRE(P.indptr[m] == n, "P_T must have exactly one entry per column");
-  const int nnz = A.indptr[n];
-  const double t_begin = now_ms();
-
-  // The fine graph does not depend on the layout: a helper thread uploads it (through the pinned
-  // staging ring when the caller's arrays are pageable) while this thread computes the layout.
-  const int64_t launches0 = ctx->launches;
-  DevBuf<int> d_I(ctx, n + 1), d_J(ctx, std::max(nnz, 1));
-  DevBuf<double> d_W;
-  if (A.data != nullptr) d_W.alloc(ctx, std::max(nnz, 1));
-  ge_status up_status = GE_OK;
-  std::string up_error;
-  std::thread uploader([&] {
-    try {
-      GE_CUDA(cudaSetDevice(ctx->device));
-      d_I.upload(ctx, A.indptr, n + 1);
-      d_J.upload(ctx, A.indices, nnz);
-      if (A.data != nullptr) d_W.upload(ctx, A.data, nnz);
-    } catch (const Fail& f) {
-      up_status = f.st;
-      up_error = ge_last_error();
-    }
-  });
-  struct Joiner {
-    std::thread& t;
-    ~Joiner() {
-      if (t.joinable()) t.join();
-    }
-  } joiner{uploader};
-
-  // host: vertex -> aggregate, segment offsets, row offsets inside the segments (O(n)); the
-  // aggregates are independent, so a few threads share them out and a prefix sum follows
-  std::vector<int> vA(std::max(n, 1), -1), rowoff(std::max(n, 1), 0), segoff((size_t)m + 1, 0);
-  {
-    const int nt = m > (1 << 16) ? 8 : 1;
-    std::vector<int> bad(nt, 0);
-    auto part = [&](int t) {
-      const int a0 = (int)((int64_t)m * t / nt), a1 = (int)((int64_t)m * (t + 1) / nt);
-      for (int a = a0; a < a1; ++a) {
-        int run = 0;
-        for (int c = P.indptr[a]; c < P.indptr[a + 1]; ++c) {
-          const int i = P.indices[c];
-          if (i < 0 || i >= n) {
-            bad[t] = 1;
-            continue;
-          }
-          vA[i] = a;
-          rowoff[i] = run;
-          run += A.indptr[i + 1] - A.indptr[i];
-        }
-        segoff[a + 1] = run;  // length for now; prefix-summed below
-      }
-    };
-    if (nt == 1) {
-      part(0);
-    } else {
-      std::vector<std::thread> pool;
-      for (int t = 0; t < nt; ++t) pool.emplace_back(part, t);
-      for (auto& th : pool) th.join();
-    }
-    bool ok = true;
-    for (int t = 0; t < nt; ++t) ok = ok && !bad[t];
-    // n entries in P_T, every one in range: all n vertices covered <=> none listed twice
-    for (int i = 0; ok && i < n; ++i) ok = vA[i] >= 0;
-    GE_REQUIRE(ok, "P_T is not a partition of the vertices");
-    for (int a = 0; a < m; ++a) segoff[a + 1] += segoff[a];
+void exclusive_scan(ge_context* ctx, const int* d_in, int n, int* d_out) {
+  const int nb = (n + kScanBlock - 1) / kScanBlock;
+  DevBuf<int> d_sums(ctx, nb + 1);
+  if (n == 0) {
+    GE_CUDA(cudaMemsetAsync(d_out, 0, sizeof(int), ctx->stream));
+    return;
   }
+  k_scan_blocks<<<nb, kScanBlock, 0, ctx->stream>>>(d_in, n, d_out, d_sums.get());
+  k_scan_sums<<<1, kScanBlock, 0, ctx->stream>>>(d_sums.get(), nb);
+  k_scan_add<<<nb, kScanBlock, 0, ctx->stream>>>(d_out, n, d_sums.get(), nb);
+  GE_CUDA(cudaGetLastError());
+  ctx->launches += 3;
+}
+
+int64_t galerkin_device(ge_context* ctx, const GalerkinInput& in, const int* segoff_host,
+                        int32_t* c_indptr, DevBuf<int>& outptr, DevBuf<int>& outcol,
+                        DevBuf<double>& outval, int64_t capacity, ge_galerkin_stats* stats,
+                        cudaEvent_t start) {
+  const int m = in.m;
+  const int nnz = segoff_host[m];
   // size classes: padded power-of-two size 32 .. 4096 in shared memory, larger in global scratch
   constexpr int kClasses = 8;  // 32, 64, ..., 4096
   std::vector<int> lists[kClasses], big;
@@ -494,7 +441,7 @@ int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P, int32_t* c_i
   std::vector<int> bigN;
   long long big_elems = 0;
   for (int a = 0; a < m; ++a) {
-    const int E = segoff[a + 1] - segoff[a];
+    const int E = segoff_host[a + 1] - segoff_host[a];
     if (E == 0) continue;  // count stays 0
     int N = 32, k = 0;
     while (N < E && N < kGalSmemMax) {
@@ -522,22 +469,11 @@ int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P, int32_t* c_i
   const int big_begin = (int)all_list.size();
   all_list.insert(all_list.end(), big.begin(), big.end());
 
-  uploader.join();  // (this thread issues CUDA calls from here on)
-  if (up_status != GE_OK) {
-    set_error("graph upload: " + up_error);
-    throw Fail{up_status};
-  }
-  DevBuf<int> d_vA(ctx, std::max(n, 1)), d_Pptr(ctx, m + 1), d_Pidx(ctx, std::max(n, 1)),
-      d_rowoff(ctx, std::max(n, 1)), d_segoff(ctx, m + 1), d_list(ctx, std::max<size_t>(all_list.size(), 1)),
-      d_count(ctx, std::max(m, 1)), d_tmpcol(ctx, std::max(nnz, 1));
+  DevBuf<int> d_list(ctx, std::max<size_t>(all_list.size(), 1)), d_count(ctx, std::max(m, 1)),
+      d_tmpcol(ctx, std::max(nnz, 1));
   DevBuf<double> d_tmpval(ctx, std::max(nnz, 1)), d_gvals(ctx, (size_t)std::max<long long>(big_elems, 1));
   DevBuf<unsigned long long> d_gkeys(ctx, (size_t)std::max<long long>(big_elems, 1));
   DevBuf<long long> d_bigoff(ctx, std::max<size_t>(bigoff.size(), 1));
-  d_vA.upload(ctx, vA.data(), n);
-  d_Pptr.upload(ctx, P.indptr, m + 1);
-  d_Pidx.upload(ctx, P.indices, n);
-  d_rowoff.upload(ctx, rowoff.data(), n);
-  d_segoff.upload(ctx, segoff.data(), m + 1);
   d_list.upload(ctx, all_list.data(), all_list.size());
   if (!bigoff.empty()) d_bigoff.upload(ctx, bigoff.data(), bigoff.size());
   d_count.zero(ctx->stream);
@@ -548,23 +484,20 @@ int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P, int32_t* c_i
     if (!verbose) return;
     GE_CUDA(cudaStreamSynchronize(ctx->stream));
     const double t = now_ms();
-    std::fprintf(stderr, "[ge] galerkin n=%d %-22s %9.3f ms\n", n, what, t - t_mark);
+    std::fprintf(stderr, "[ge] galerkin n=%d %-22s %9.3f ms\n", in.n, what, t - t_mark);
     t_mark = t;
   };
   lap("layout + upload");
-  cudaEvent_t ev0, ev1;
-  GE_CUDA(cudaEventCreate(&ev0));
-  GE_CUDA(cudaEventCreate(&ev1));
-  GE_CUDA(cudaEventRecord(ev0, ctx->stream));
+  if (start) GE_CUDA(cudaEventRecord(start, ctx->stream));
   GalArgs g;
-  g.I = d_I.get();
-  g.J = d_J.get();
-  g.W = A.data != nullptr ? d_W.get() : nullptr;
-  g.vA = d_vA.get();
-  g.Pptr = d_Pptr.get();
-  g.Pidx = d_Pidx.get();
-  g.rowoff = d_rowoff.get();
-  g.segoff = d_segoff.get();
+  g.I = in.I;
+  g.J = in.J;
+  g.W = in.W;
+  g.vA = in.vA;
+  g.Pptr = in.Pptr;
+  g.Pidx = in.Pidx;
+  g.rowoff = in.rowoff;
+  g.segoff = in.segoff;
   g.count = d_count.get();
   g.tmpcol = d_tmpcol.get();
   g.tmpval = d_tmpval.get();
@@ -638,47 +571,159 @@ int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P, int32_t* c_i
     lap("big: reduce");
   }
   // row lengths -> exclusive scan on the device -> final offsets (nnz(A_c) <= nnz(A) < 2^31)
-  const int nb = (m + kScanBlock - 1) / kScanBlock;
-  DevBuf<int> d_outptr(ctx, m + 1), d_sums(ctx, nb + 1);
+  outptr.alloc(ctx, (size_t)m + 1);
+  int total32 = 0;
   if (m > 0) {
-    k_scan_blocks<<<nb, kScanBlock, 0, ctx->stream>>>(d_count.get(), m, d_outptr.get(), d_sums.get());
-    k_scan_sums<<<1, kScanBlock, 0, ctx->stream>>>(d_sums.get(), nb);
-    k_scan_add<<<nb, kScanBlock, 0, ctx->stream>>>(d_outptr.get(), m, d_sums.get(), nb);
-    GE_CUDA(cudaGetLastError());
-    ctx->launches += 3;
-    d_outptr.download(ctx, c_indptr, m + 1);
-    GE_CUDA(cudaStreamSynchronize(ctx->stream));
+    exclusive_scan(ctx, d_count.get(), m, outptr.get());
+    if (c_indptr) {
+      outptr.download(ctx, c_indptr, (size_t)m + 1);
+      GE_CUDA(cudaStreamSynchronize(ctx->stream));
+      total32 = c_indptr[m];
+    } else {
+      GE_CUDA(cudaMemcpyAsync(&total32, outptr.get() + m, sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+      GE_CUDA(cudaStreamSynchronize(ctx->stream));
+    }
   } else {
-    c_indptr[0] = 0;
+    outptr.zero(ctx->stream);
+    if (c_indptr) c_indptr[0] = 0;
   }
   lap("scan + row pointers");
-  const int64_t total = c_indptr[m];
+  const int64_t total = total32;
   if (total <= capacity && total > 0) {
-    GE_REQUIRE(c_indices && c_data, "null output arrays");
-    DevBuf<int> d_outcol(ctx, (size_t)total);
-    DevBuf<double> d_outval(ctx, (size_t)total);
+    outcol.alloc(ctx, (size_t)total);
+    outval.alloc(ctx, (size_t)total);
     const unsigned grid = (unsigned)(((int64_t)m * 32 + 255) / 256);
-    k_gal_compact<<<grid, 256, 0, ctx->stream>>>(d_segoff.get(), d_outptr.get(), m, d_tmpcol.get(),
-                                                 d_tmpval.get(), d_outcol.get(), d_outval.get());
+    k_gal_compact<<<grid, 256, 0, ctx->stream>>>(in.segoff, outptr.get(), m, d_tmpcol.get(),
+                                                 d_tmpval.get(), outcol.get(), outval.get());
     GE_CUDA(cudaGetLastError());
     ctx->launches++;
-    GE_CUDA(cudaEventRecord(ev1, ctx->stream));
+  }
+  if (stats) {
+    stats->segments_shared = big_begin;
+    stats->segments_global = (int64_t)big.size();
+    stats->nnz_out = total;
+  }
+  return total;
+}
+
+// Returns nnz(A_c); fills c_indptr always, c_indices / c_data when capacity suffices.
+int64_t galerkin(ge_context* ctx, const ge_csr& A, const ge_csr& P, int32_t* c_indptr,
+                 int32_t* c_indices, double* c_data, int64_t capacity, ge_galerkin_stats* stats) {
+  const int n = A.rows, m = P.rows;
+  GE_REQUIRE(A.rows == A.cols, "A must be square");
+  GE_REQUIRE(P.cols == n, "P_T.cols != A.rows");
+  GE_REQUIRE(P.indptr[m] == n, "P_T must have exactly one entry per column");
+  const int nnz = A.indptr[n];
+  const double t_begin = now_ms();
+
+  // The fine graph does not depend on the layout: a helper thread uploads it (through the pinned
+  // staging ring when the caller's arrays are pageable) while this thread computes the layout.
+  const int64_t launches0 = ctx->launches;
+  DevBuf<int> d_I(ctx, n + 1), d_J(ctx, std::max(nnz, 1));
+  DevBuf<double> d_W;
+  if (A.data != nullptr) d_W.alloc(ctx, std::max(nnz, 1));
+  ge_status up_status = GE_OK;
+  std::string up_error;
+  std::thread uploader([&] {
+    try {
+      GE_CUDA(cudaSetDevice(ctx->device));
+      d_I.upload(ctx, A.indptr, n + 1);
+      d_J.upload(ctx, A.indices, nnz);
+      if (A.data != nullptr) d_W.upload(ctx, A.data, nnz);
+    } catch (const Fail& f) {
+      up_status = f.st;
+      up_error = ge_last_error();
+    }
+  });
+  struct Joiner {
+    std::thread& t;
+    ~Joiner() {
+      if (t.joinable()) t.join();
+    }
+  } joiner{uploader};
+
+  // host: vertex -> aggregate, segment offsets, row offsets inside the segments (O(n)); the
+  // aggregates are independent, so a few threads share them out and a prefix sum follows
+  std::vector<int> vA(std::max(n, 1), -1), rowoff(std::max(n, 1), 0), segoff((size_t)m + 1, 0);
+  {
+    const int nt = m > (1 << 16) ? 8 : 1;
+    std::vector<int> bad(nt, 0);
+    auto part = [&](int t) {
+      const int a0 = (int)((int64_t)m * t / nt), a1 = (int)((int64_t)m * (t + 1) / nt);
+      for (int a = a0; a < a1; ++a) {
+        int run = 0;
+        for (int c = P.indptr[a]; c < P.indptr[a + 1]; ++c) {
+          const int i = P.indices[c];
+          if (i < 0 || i >= n) {
+            bad[t] = 1;
+            continue;
+          }
+          vA[i] = a;
+          rowoff[i] = run;
+          run += A.indptr[i + 1] - A.indptr[i];
+        }
+        segoff[a + 1] = run;  // length for now; prefix-summed below
+      }
+    };
+    if (nt == 1) {
+      part(0);
+    } else {
+      std::vector<std::thread> pool;
+      for (int t = 0; t < nt; ++t) pool.emplace_back(part, t);
+      for (auto& th : pool) th.join();
+    }
+    bool ok = true;
+    for (int t = 0; t < nt; ++t) ok = ok && !bad[t];
+    // n entries in P_T, every one in range: all n vertices covered <=> none listed twice
+    for (int i = 0; ok && i < n; ++i) ok = vA[i] >= 0;
+    GE_REQUIRE(ok, "P_T is not a partition of the vertices");
+    for (int a = 0; a < m; ++a) segoff[a + 1] += segoff[a];
+  }
+
+  uploader.join();  // (this thread issues CUDA calls from here on)
+  if (up_status != GE_OK) {
+    set_error("graph upload: " + up_error);
+    throw Fail{up_status};
+  }
+  DevBuf<int> d_vA(ctx, std::max(n, 1)), d_Pptr(ctx, m + 1), d_Pidx(ctx, std::max(n, 1)),
+      d_rowoff(ctx, std::max(n, 1)), d_segoff(ctx, m + 1);
+  d_vA.upload(ctx, vA.data(), n);
+  d_Pptr.upload(ctx, P.indptr, m + 1);
+  d_Pidx.upload(ctx, P.indices, n);
+  d_rowoff.upload(ctx, rowoff.data(), n);
+  d_segoff.upload(ctx, segoff.data(), m + 1);
+
+  cudaEvent_t ev0, ev1;
+  GE_CUDA(cudaEventCreate(&ev0));
+  GE_CUDA(cudaEventCreate(&ev1));
+  GalerkinInput in;
+  in.n = n;
+  in.m = m;
+  in.I = d_I.get();
+  in.J = d_J.get();
+  in.W = A.data != nullptr ? d_W.get() : nullptr;
+  in.vA = d_vA.get();
+  in.Pptr = d_Pptr.get();
+  in.Pidx = d_Pidx.get();
+  in.rowoff = d_rowoff.get();
+  in.segoff = d_segoff.get();
+  DevBuf<int> d_outptr, d_outcol;
+  DevBuf<double> d_outval;
+  const int64_t total = galerkin_device(ctx, in, segoff.data(), c_indptr, d_outptr, d_outcol, d_outval,
+                                        capacity, stats, ev0);
+  GE_CUDA(cudaEventRecord(ev1, ctx->stream));
+  if (total <= capacity && total > 0) {
+    GE_REQUIRE(c_indices && c_data, "null output arrays");
     d_outcol.download(ctx, c_indices, (size_t)total);
     d_outval.download(ctx, c_data, (size_t)total);
-    GE_CUDA(cudaStreamSynchronize(ctx->stream));
-  } else {
-    GE_CUDA(cudaEventRecord(ev1, ctx->stream));
-    GE_CUDA(cudaStreamSynchronize(ctx->stream));
   }
+  GE_CUDA(cudaStreamSynchronize(ctx->stream));
   if (stats) {
     float ms = 0;
     GE_CUDA(cudaEventElapsedTime(&ms, ev0, ev1));
     stats->device_ms = ms;  // kernels + the row-length round trip
     stats->total_ms = now_ms() - t_begin;
     stats->kernel_launches = ctx->launches - launches0;
-    stats->segments_shared = big_begin;
-    stats->segments_global = (int64_t)big.size();
-    stats->nnz_out = total;
   }
   cudaEventDestroy(ev0);
   cudaEventDestroy(ev1);

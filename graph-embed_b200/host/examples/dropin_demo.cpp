@@ -61,14 +61,40 @@ int flat_on_gpus(int gpus, int dimension) {
   return 0;
 }
 
+// `--coarsen`: graph -> hierarchy built on the device (ge_b200::coarsen) -> partition::embed.
+int coarsen_then_embed(int nx, int dimension) {
+  ge_b200::options().seed = 3;
+  std::vector<SparseMatrix> As;
+  linalgcpp::Timer timer(linalgcpp::Timer::Start::True);
+  const std::vector<SparseMatrix> hierarchy = ge_b200::coarsen(grid(nx, nx), 0.25, 64, &As);
+  timer.Click();
+  std::cout << "coarsen: " << hierarchy.size() << " levels in " << timer[0] << "s:";
+  for (const auto& A : As) std::cout << " " << A.Rows();
+  std::cout << std::endl;
+  linalgcpp::Timer t2(linalgcpp::Timer::Start::True);
+  std::vector<std::vector<double>> coords = partition::embed(As, hierarchy, dimension);
+  t2.Click();
+  std::cout << "embedded! in time " << t2[0] << "s" << std::endl;
+  for (size_t i = 0; i < coords.size(); i++)
+    for (int k = 0; k < dimension; k++)
+      if (std::isnan(coords[i][k])) {
+        std::cerr << "NaN at vertex " << i << std::endl;
+        return 1;
+      }
+  return coords.size() == static_cast<size_t>(nx) * nx ? 0 : 2;
+}
+
 int main(int argc, char** argv) {
   std::string outdir;  // --out DIR: write the layout and the plot inputs like examples/embedder.cpp:230-289
-  for (int a = 1; a + 1 < argc; ++a) {
-    if (std::string(argv[a]) == "--gpus") return flat_on_gpus(std::atoi(argv[a + 1]), 2);
-    if (std::string(argv[a]) == "--out") outdir = argv[a + 1];
+  bool coarsen = false;
+  for (int a = 1; a < argc; ++a) {
+    if (a + 1 < argc && std::string(argv[a]) == "--gpus") return flat_on_gpus(std::atoi(argv[a + 1]), 2);
+    if (a + 1 < argc && std::string(argv[a]) == "--out") outdir = argv[a + 1];
+    if (std::string(argv[a]) == "--coarsen") coarsen = true;
   }
   int nx = argc > 1 ? std::atoi(argv[1]) : 64, ny = nx;
   const int dimension = argc > 2 ? std::atoi(argv[2]) : 2;
+  if (coarsen) return coarsen_then_embed(nx, dimension);
   std::vector<SparseMatrix> As = {grid(nx, ny)}, hierarchy;
   while (nx * ny > 40) {
     hierarchy.push_back(blocks(nx, ny));

@@ -93,6 +93,47 @@ inline SparseMatrix galerkin(const SparseMatrix& A, const SparseMatrix& P_T) {
   return SparseMatrix(std::move(indptr), std::move(indices), std::move(data), P_T.Rows(), P_T.Rows());
 }
 
+// The multilevel hierarchy built on the device (ge_coarsen: random-mate matching, NOT the
+// reference's partitioner).  Returns the P_T of every level, the shape partition::partition
+// returns; As (when not null) receives the graphs {A, A_1, ..., A_L}, ready for partition::embed.
+inline std::vector<SparseMatrix> coarsen(const SparseMatrix& A, double coarseningFactor, int minCoarse,
+                                         std::vector<SparseMatrix>* As = nullptr) {
+  const ge_csr a = view(A);
+  ge_coarsen_options opt;
+  ge_coarsen_options_default(&opt);
+  opt.coarsening_factor = coarseningFactor;
+  opt.min_coarse = minCoarse;
+  opt.seed = options().seed;
+  ge_hierarchy* h = nullptr;
+  check(ge_coarsen(default_context(), &a, &opt, &h, nullptr));
+  struct Owner {
+    ge_hierarchy* h;
+    ~Owner() { ge_hierarchy_destroy(h); }
+  } owner{h};
+  auto copy = [](const ge_csr& c) {
+    const int64_t nnz = c.nnz;
+    return SparseMatrix(std::vector<int>(c.indptr, c.indptr + c.rows + 1),
+                        std::vector<int>(c.indices, c.indices + nnz), std::vector<double>(c.data, c.data + nnz),
+                        c.rows, c.cols);
+  };
+  const int L = ge_hierarchy_levels(h);
+  std::vector<SparseMatrix> P_Ts;
+  if (As) {
+    As->clear();
+    As->push_back(A);
+  }
+  for (int l = 0; l < L; ++l) {
+    ge_csr c;
+    check(ge_hierarchy_aggregation(h, l, &c));
+    P_Ts.push_back(copy(c));
+    if (As) {
+      check(ge_hierarchy_graph(h, l + 1, &c));
+      As->push_back(copy(c));
+    }
+  }
+  return P_Ts;
+}
+
 }  // namespace ge_b200
 
 #endif

@@ -210,6 +210,49 @@ ge_status ge_galerkin(ge_context* ctx, const ge_csr* A, const ge_csr* P_T, int32
                       int32_t* c_indices, double* c_data, int64_t capacity, int64_t* nnz_out,
                       ge_galerkin_stats* stats /* may be NULL */);
 
+/* ---- multilevel hierarchy on the device ------------------------------------------------------ */
+/* Random-mate matching, level by level: the stand-in hierarchy generator of the project
+ * (graphs.coarsen) made deterministic.  This is NOT the reference's partitioner
+ * (src/partitioner.cpp:1550-1893); it is an additional way to go from a graph to the input of
+ * ge_embed.  Each round, a counter-based hash H(tag, v) of (seed, level, round) splits the vertices
+ * into heads and tails; every tail picks the head neighbour with the largest w_ij / (k_i k_j)
+ * (k = weighted degree, self-loop included), ties to the smaller hash then the smaller id; when
+ * more tails found a head than the level still needs, the ones with the smallest H(1, i) merge.
+ * The round's graph is contracted with the Galerkin product of ge_galerkin.  A level ends at
+ * max(floor(coarsening_factor * n), min_coarse) vertices or when no tail finds a head; the
+ * hierarchy ends after max_levels levels, at min_coarse vertices, or at a level that merged nothing.
+ * The result is a pure function of (A, options); tests/coarsen_restatement.py restates it on
+ * the host. */
+typedef struct ge_coarsen_options {
+  double coarsening_factor; /* 0.25; in (0, 1] */
+  int32_t min_coarse;       /* 64; >= 1 */
+  int32_t max_levels;       /* 32; >= 0 */
+  uint32_t seed;            /* 0; every value, 0 included, is an ordinary seed */
+} ge_coarsen_options;
+
+typedef struct ge_coarsen_stats {
+  double total_ms;         /* whole call: upload, every round, download of the levels */
+  double device_ms;        /* CUDA events from the first kernel to the end of the download */
+  int64_t rounds;          /* matching rounds, all levels */
+  int64_t kernel_launches; /* one CUB sort / select call counts as one launch */
+} ge_coarsen_stats;
+
+typedef struct ge_hierarchy ge_hierarchy; /* host copy of the levels, owned by the handle */
+
+void ge_coarsen_options_default(ge_coarsen_options* opt);
+/* A: n x n CSR (data NULL = unit weights), finite weights.  On a multi-device context the call runs
+ * on the first device.  *out receives a new handle (free it with ge_hierarchy_destroy); stats may
+ * be NULL. */
+ge_status ge_coarsen(ge_context* ctx, const ge_csr* A, const ge_coarsen_options* opt,
+                     ge_hierarchy** out, ge_coarsen_stats* stats);
+/* Number of levels L: the hierarchy has graphs As[0..L] (As[0] = A) and aggregations P_T[0..L-1]. */
+int32_t ge_hierarchy_levels(const ge_hierarchy* h);
+/* View of As[l], l = 1..L: columns ascending per row, diagonal entries included. */
+ge_status ge_hierarchy_graph(const ge_hierarchy* h, int32_t l, ge_csr* out);
+/* View of P_T[l], l = 0..L-1 (As[l+1].rows x As[l].rows, members ascending per row, unit data). */
+ge_status ge_hierarchy_aggregation(const ge_hierarchy* h, int32_t l, ge_csr* out);
+void ge_hierarchy_destroy(ge_hierarchy* h);
+
 /* The reference's random stream: count draws of uniform_real_distribution<double>(-1,1) over
  * std::mt19937(seed) (include/forceatlas.hpp:104-108). */
 void ge_reference_uniform(uint32_t seed, int64_t count, double* out);
