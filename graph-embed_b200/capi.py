@@ -75,7 +75,7 @@ SYMBOLS = [
     "ge_context_create_multi", "ge_context_device_count",
     "ge_flat_symmetric_pass_share", "ge_embed_aggregate_ranges", "ge_embed_aggregate_owners",
     "ge_coarsen_options_default", "ge_coarsen", "ge_hierarchy_levels", "ge_hierarchy_graph",
-    "ge_hierarchy_aggregation", "ge_hierarchy_destroy",
+    "ge_hierarchy_aggregation", "ge_hierarchy_destroy", "ge_largest_component", "ge_layout_graph",
 ]
 
 _lib = None
@@ -139,6 +139,12 @@ class CoarsenOptions(C.Structure):
 class CoarsenStats(C.Structure):
     _fields_ = [("total_ms", C.c_double), ("device_ms", C.c_double), ("rounds", C.c_int64),
                 ("kernel_launches", C.c_int64)]
+
+
+class LayoutStats(C.Structure):
+    _fields_ = [("total_ms", C.c_double), ("components_ms", C.c_double), ("coarsen_ms", C.c_double),
+                ("embed_ms", C.c_double), ("components", C.c_int64), ("levels", C.c_int32),
+                ("h2d_bytes", C.c_double), ("d2h_bytes", C.c_double), ("kernel_launches", C.c_int64)]
 
 
 def _csr_copy(c, with_data=True):
@@ -380,6 +386,51 @@ class Context:
         finally:
             lib().ge_hierarchy_destroy(h)
         return As, Ps, {f: getattr(st, f) for f, _ in st._fields_}
+
+    def largest_component(self, A):
+        """ge_largest_component -> (B, vertices, components): B = A[vertices][:, vertices] as scipy CSR,
+        vertices the kept original ids (ascending), components the number of components of A."""
+        import scipy.sparse as sp
+        a = CsrView(sp.csr_matrix(A))
+        n = A.shape[0]
+        cap = max(int(a.indptr[-1]), 1)
+        vert = np.zeros(max(n, 1), dtype=np.int32)
+        ptr = np.zeros(n + 1, dtype=np.int32)
+        idx = np.zeros(cap, dtype=np.int32)
+        val = np.zeros(cap)
+        n_out, nnz, comps = C.c_int32(), C.c_int64(), C.c_int64()
+        _check(lib().ge_largest_component(self.h, a.ref(), _ptr(vert, _pi), C.byref(n_out), _ptr(ptr, _pi),
+                                          _ptr(idx, _pi), _ptr(val, _pd), C.c_int64(cap), C.byref(nnz),
+                                          C.byref(comps)))
+        k, e = int(n_out.value), int(nnz.value)
+        B = sp.csr_matrix((val[:e].copy(), idx[:e].copy(), ptr[:k + 1].copy()), shape=(k, k))
+        return B, vert[:k].copy(), int(comps.value)
+
+    def layout(self, A, dim, coarsening_factor=0.25, min_coarse=64, max_levels=32, coarsen_seed=0, seed=0,
+               largest_component=True, precision=GE_F64, coarse_iterations=100000, level_iterations=100,
+               verbose=False):
+        """ge_layout_graph: [largest component] -> ge_coarsen -> ge_embed in one call ->
+        (coords [n x dim], vertices [n] original ids of the rows, stats)."""
+        import scipy.sparse as sp
+        a = CsrView(sp.csr_matrix(A))
+        copt = CoarsenOptions()
+        lib().ge_coarsen_options_default(C.byref(copt))
+        copt.coarsening_factor, copt.min_coarse = float(coarsening_factor), int(min_coarse)
+        copt.max_levels, copt.seed = int(max_levels), int(coarsen_seed)
+        eopt = EmbedOptions()
+        lib().ge_embed_options_default(C.byref(eopt))
+        eopt.seed, eopt.precision, eopt.verbose = int(seed), int(precision), int(verbose)
+        eopt.coarse_iterations, eopt.level_iterations = int(coarse_iterations), int(level_iterations)
+        n = A.shape[0]
+        out = np.zeros((max(n, 1), dim))
+        vert = np.zeros(max(n, 1), dtype=np.int32)
+        n_out = C.c_int32()
+        st = LayoutStats()
+        _check(lib().ge_layout_graph(self.h, a.ref(), int(dim), int(bool(largest_component)), C.byref(copt),
+                                     C.byref(eopt), _ptr(out, _pd), _ptr(vert, _pi), C.byref(n_out),
+                                     C.byref(st)))
+        k = int(n_out.value)
+        return out[:k].copy(), vert[:k].copy(), {f: getattr(st, f) for f, _ in st._fields_}
 
     def flat_plan(self, A, dim, params, rows=None, symmetric=None):
         """rows=(r0, r1): ordered row-block plan; symmetric=(rank, world): that rank's plan of a

@@ -514,6 +514,16 @@ struct EmbedRun {
   const ge_csr* Ps;
   ge_embed_options opt;
   ge_embed_stats st{};
+  // ge_layout_graph: the graphs of levels 0..L-1 are already on device 0 and As[l] carries their row
+  // pointers only.  Device 0 takes their buffers over; another device copies them from device 0
+  // (dev_src: their addresses, which stay valid while device 0 owns them).
+  DeviceHierarchy* on_device = nullptr;
+  struct DevSrc {
+    const int* I;
+    const int* J;
+    const double* W;
+  };
+  std::vector<DevSrc> dev_src;
 
   // Per device: the level graphs + slot layouts (inputs that do not depend on any result: a helper
   // thread uploads the large ones on the device's copy stream while the coarsest-level solve, one
@@ -567,14 +577,48 @@ struct EmbedRun {
     }
   }
 
-  static void upload_graph(ge_context* c, const ge_csr& A, PrefetchedGraph& g) {
+  void adopt_device_levels() {
+    if (on_device == nullptr) return;
+    for (int l = 0; l < L; ++l) {
+      const DevGraph& G = *on_device->graphs[l];
+      dev_src.push_back(DevSrc{G.I.get(), G.J.get(), G.w()});
+    }
+  }
+
+  // Level l's graph on device d (context c): from the host arrays, or from the device hierarchy.
+  void fetch_graph(ge_context* c, int d, int l, PrefetchedGraph& g) {
+    const ge_csr& A = As[l];
+    if (on_device == nullptr) {
+      g.I.alloc(c, A.rows + 1);
+      g.J.alloc(c, (size_t)std::max<int64_t>(A.nnz, 1));
+      g.I.upload(c, A.indptr, A.rows + 1);
+      g.J.upload(c, A.indices, (size_t)A.nnz);
+      if (A.data != nullptr) {
+        g.Dw.alloc(c, (size_t)std::max<int64_t>(A.nnz, 1));
+        g.Dw.upload(c, A.data, (size_t)A.nnz);
+      }
+      return;
+    }
+    if (d == 0) {
+      DevGraph& G = *on_device->graphs[l];
+      g.I = std::move(G.I);
+      g.J = std::move(G.J);
+      g.Dw = std::move(G.W);
+      return;
+    }
+    const DevSrc& src = dev_src[l];
     g.I.alloc(c, A.rows + 1);
     g.J.alloc(c, (size_t)std::max<int64_t>(A.nnz, 1));
-    g.I.upload(c, A.indptr, A.rows + 1);
-    g.J.upload(c, A.indices, (size_t)A.nnz);
-    if (A.data != nullptr) {
+    GE_CUDA(cudaMemcpyPeerAsync(g.I.get(), c->device, src.I, ctx->device, sizeof(int) * ((size_t)A.rows + 1),
+                                c->stream));
+    if (A.nnz)
+      GE_CUDA(cudaMemcpyPeerAsync(g.J.get(), c->device, src.J, ctx->device, sizeof(int) * (size_t)A.nnz,
+                                  c->stream));
+    if (src.W != nullptr) {
       g.Dw.alloc(c, (size_t)std::max<int64_t>(A.nnz, 1));
-      g.Dw.upload(c, A.data, (size_t)A.nnz);
+      if (A.nnz)
+        GE_CUDA(cudaMemcpyPeerAsync(g.Dw.get(), c->device, src.W, ctx->device, sizeof(double) * (size_t)A.nnz,
+                                    c->stream));
     }
   }
 
@@ -601,7 +645,7 @@ struct EmbedRun {
             if (A.nnz < kPrefetchMinNnz) continue;
             if (d != 0 && dev->a1[l] <= dev->a0[l]) continue;
             std::unique_ptr<PrefetchedGraph> g(new PrefetchedGraph);
-            upload_graph(&side, A, *g);
+            fetch_graph(&side, (int)d, l, *g);
             g->layout = sharded[l] ? make_level_layout(&side, Ps[l], A.rows, 0, -1, d == 0, &dev->owned[l])
                                    : make_level_layout(&side, Ps[l], A.rows, dev->a0[l], dev->a1[l], d == 0);
             GE_CUDA(cudaEventCreateWithFlags(&g->ready, cudaEventDisableTiming));
@@ -644,6 +688,11 @@ struct EmbedRun {
       // the prefetched buffers were allocated on the copy stream: nothing on the main stream may
       // still read them when they are returned to the pool
       cudaStreamSynchronize(dev.ctx->stream);
+      if (dev.ctx->copy_stream) cudaStreamSynchronize(dev.ctx->copy_stream);
+    }
+    // (device 0's level graphs are the source of the other devices' copies: freed after every sync)
+    for (auto& dev : devs) {
+      cudaSetDevice(dev.ctx->device);
       dev.pre.clear();
     }
     cudaSetDevice(ctx->device);
@@ -656,7 +705,7 @@ struct EmbedRun {
     if (dev.pre[l]) return dev.pre[l].get();
     const ge_csr& A = As[l];
     std::unique_ptr<PrefetchedGraph> g(new PrefetchedGraph);
-    upload_graph(dev.ctx, A, *g);
+    fetch_graph(dev.ctx, d, l, *g);
     g->layout = sharded[l] ? make_level_layout(dev.ctx, Ps[l], A.rows, 0, -1, d == 0, &dev.owned[l])
                            : make_level_layout(dev.ctx, Ps[l], A.rows, dev.a0[l], dev.a1[l], d == 0);
     GE_CUDA(cudaEventCreateWithFlags(&g->ready, cudaEventDisableTiming));
@@ -687,6 +736,15 @@ struct EmbedRun {
     // coarsest level too large for the device's event arrays)
     const double t0 = now_ms();
     std::vector<double> x((size_t)m * dim), r(m, 0.0), xc, rc;
+    std::vector<int> cols;
+    ge_csr Ak = As[k];
+    if (!base && Ak.indices == nullptr) {  // a level on the device only: its columns come down
+      const PrefetchedGraph* g = graph(0, k);
+      GE_CUDA(cudaStreamWaitEvent(ctx->stream, g->ready, 0));
+      cols.resize((size_t)Ak.nnz);
+      g->J.download(ctx, cols.data(), cols.size());
+      Ak.indices = cols.data();
+    }
     d0.dx[k].download(ctx, x.data(), x.size());
     if (!base) {
       const int mc = As[k + 1].rows;
@@ -697,7 +755,7 @@ struct EmbedRun {
     }
     GE_CUDA(cudaStreamSynchronize(ctx->stream));
     if (base) level_radii(m, dim, x.data(), r.data(), nullptr, nullptr, nullptr, nullptr);
-    else level_radii(m, dim, x.data(), r.data(), &As[k], &Ps[k], xc.data(), rc.data());
+    else level_radii(m, dim, x.data(), r.data(), &Ak, &Ps[k], xc.data(), rc.data());
     d0.dx[k].upload(ctx, x.data(), x.size());
     d0.dr[k].upload(ctx, r.data(), r.size());
     GE_CUDA(cudaStreamSynchronize(ctx->stream));
@@ -841,6 +899,37 @@ struct EmbedRun {
   }
 };
 
+// ge_embed's driver; on_device: ge_layout_graph's hierarchy (see EmbedRun::on_device)
+void embed_levels(ge_context* ctx, int L, const ge_csr* As, const ge_csr* P_Ts, int dim,
+                  const ge_embed_options* opt, double* coords_out, double* r_A_out, double* coords_A_out,
+                  ge_embed_stats* stats, DeviceHierarchy* on_device) {
+  EmbedRun run;
+  run.ctx = ctx;
+  run.L = L;
+  run.dim = dim;
+  run.As = As;
+  run.Ps = P_Ts;
+  run.on_device = on_device;
+  if (opt) run.opt = *opt;
+  else ge_embed_options_default(&run.opt);
+  const int64_t launches0 = ctx->launches;
+  const double h0 = ctx->h2d_bytes, d0 = ctx->d2h_bytes;
+  ctx->grid_tier_ms = 0;
+  ctx->radii_ms = 0;
+  const double t0 = now_ms();
+  run.adopt_device_levels();
+  run.plan_ranges();
+  run.start_prefetch();
+  run.run(coords_out, r_A_out, coords_A_out);
+  run.st.total_ms = now_ms() - t0;
+  run.st.kernel_launches = ctx->launches - launches0;
+  run.st.h2d_bytes = ctx->h2d_bytes - h0;
+  run.st.d2h_bytes = ctx->d2h_bytes - d0;
+  run.st.grid_tier_ms = ctx->grid_tier_ms;
+  run.st.device_radii_ms = ctx->radii_ms;
+  if (stats) *stats = run.st;
+}
+
 template <typename F>
 ge_status guarded(F&& body) {
   try {
@@ -854,6 +943,16 @@ ge_status guarded(F&& body) {
   } catch (const std::exception& e) {
     set_error(e.what());
     return GE_ERR_INVALID;
+  }
+}
+
+// GE_ERR_NO_DEVICE without a usable device, before any argument is looked at
+void require_device() {
+  int count = 0;
+  if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
+    cudaGetLastError();
+    set_error("no usable CUDA device (this library has no CPU fallback)");
+    throw Fail{GE_ERR_NO_DEVICE};
   }
 }
 
@@ -1066,29 +1165,7 @@ ge_status ge_embed(ge_context* ctx, int n_levels, const ge_csr* As, const ge_csr
       GE_REQUIRE(As[l].rows == P_Ts[l].cols, "As[l].Rows() != P_Ts[l].Cols()");
       GE_REQUIRE(As[l + 1].rows == P_Ts[l].rows, "As[l+1].Rows() != P_Ts[l].Rows()");
     }
-    EmbedRun run;
-    run.ctx = ctx;
-    run.L = n_levels;
-    run.dim = dim;
-    run.As = As;
-    run.Ps = P_Ts;
-    if (opt) run.opt = *opt;
-    else ge_embed_options_default(&run.opt);
-    const int64_t launches0 = ctx->launches;
-    const double h0 = ctx->h2d_bytes, d0 = ctx->d2h_bytes;
-    ctx->grid_tier_ms = 0;
-    ctx->radii_ms = 0;
-    const double t0 = now_ms();
-    run.plan_ranges();
-    run.start_prefetch();
-    run.run(coords_out, r_A_out, coords_A_out);
-    run.st.total_ms = now_ms() - t0;
-    run.st.kernel_launches = ctx->launches - launches0;
-    run.st.h2d_bytes = ctx->h2d_bytes - h0;
-    run.st.d2h_bytes = ctx->d2h_bytes - d0;
-    run.st.grid_tier_ms = ctx->grid_tier_ms;
-    run.st.device_radii_ms = ctx->radii_ms;
-    if (stats) *stats = run.st;
+    embed_levels(ctx, n_levels, As, P_Ts, dim, opt, coords_out, r_A_out, coords_A_out, stats, nullptr);
   });
 }
 
@@ -1204,18 +1281,177 @@ ge_status ge_coarsen(ge_context* ctx, const ge_csr* A, const ge_coarsen_options*
   return guarded([&] {
     GE_REQUIRE(out != nullptr, "out is null");
     *out = nullptr;
-    int count = 0;
-    if (cudaGetDeviceCount(&count) != cudaSuccess || count == 0) {
-      cudaGetLastError();
-      set_error("no usable CUDA device (this library has no CPU fallback)");
-      throw Fail{GE_ERR_NO_DEVICE};
-    }
+    require_device();
     require_ctx(ctx);  // a multi-device context: its first device
     check_csr(A, "A");
     GE_REQUIRE(opt != nullptr, "options are null");
     std::unique_ptr<ge_hierarchy> h(new ge_hierarchy);
     coarsen(ctx, *A, *opt, *h, stats);
     *out = h.release();
+  });
+}
+
+ge_status ge_largest_component(ge_context* ctx, const ge_csr* A, int32_t* vertices, int32_t* n_out,
+                               int32_t* c_indptr, int32_t* c_indices, double* c_data, int64_t capacity,
+                               int64_t* nnz_out, int64_t* components) {
+  return guarded([&] {
+    require_device();
+    require_ctx(ctx);  // a multi-device context: its first device
+    check_csr(A, "A");
+    GE_REQUIRE(A->rows == A->cols, "A must be square");
+    GE_REQUIRE(vertices && n_out && c_indptr && nnz_out, "null argument");
+    DevGraph G, C;
+    DevBuf<int> kept;
+    upload_graph(ctx, *A, G);
+    check_graph(ctx, G);
+    const int64_t ncomp = largest_component_device(ctx, G, C, kept);
+    if (components) *components = ncomp;
+    if (ncomp <= 1) {  // connected (or empty): A itself
+      const int n = A->rows;
+      *n_out = n;
+      for (int v = 0; v < n; ++v) vertices[v] = v;
+      std::memcpy(c_indptr, A->indptr, sizeof(int32_t) * ((size_t)n + 1));
+      *nnz_out = A->nnz;
+      GE_REQUIRE(A->nnz <= capacity, "output capacity too small (see *nnz_out)");
+      GE_REQUIRE(A->nnz == 0 || (c_indices && c_data), "c_indices / c_data are null");
+      if (A->nnz) std::memcpy(c_indices, A->indices, sizeof(int32_t) * (size_t)A->nnz);
+      if (A->data) std::memcpy(c_data, A->data, sizeof(double) * (size_t)A->nnz);
+      else std::fill(c_data, c_data + A->nnz, 1.0);
+      return;
+    }
+    *n_out = C.n;
+    *nnz_out = C.nnz;
+    kept.download(ctx, vertices, (size_t)C.n);
+    C.I.download(ctx, c_indptr, (size_t)C.n + 1);
+    if (C.nnz <= capacity) {
+      GE_REQUIRE(C.nnz == 0 || (c_indices && c_data), "c_indices / c_data are null");
+      C.J.download(ctx, c_indices, (size_t)C.nnz);
+      C.W.download(ctx, c_data, (size_t)C.nnz);
+    }
+    GE_CUDA(cudaStreamSynchronize(ctx->stream));
+    GE_REQUIRE(C.nnz <= capacity, "output capacity too small (see *nnz_out)");
+  });
+}
+
+ge_status ge_layout_graph(ge_context* ctx, const ge_csr* A, int dim, int32_t largest_component,
+                          const ge_coarsen_options* copt, const ge_embed_options* eopt, double* coords_out,
+                          int32_t* vertices_out, int32_t* n_out, ge_layout_stats* stats) {
+  return guarded([&] {
+    require_device();
+    require_ctx(ctx);
+    check_csr(A, "A");
+    GE_REQUIRE(A->rows == A->cols, "A must be square");
+    GE_REQUIRE(coords_out && n_out, "null argument");
+    ge_coarsen_options co;
+    if (copt) co = *copt;
+    else ge_coarsen_options_default(&co);
+    check_coarsen_options(co);
+    ge_layout_stats st;
+    std::memset(&st, 0, sizeof(st));
+    const double t0 = now_ms();
+    const int64_t launches0 = ctx->launches;
+    const double h0 = ctx->h2d_bytes, d0 = ctx->d2h_bytes;
+    cudaEvent_t ev[4];
+    for (auto& e : ev) GE_CUDA(cudaEventCreate(&e));
+    struct Events {
+      cudaEvent_t* e;
+      ~Events() {
+        for (int i = 0; i < 4; ++i) cudaEventDestroy(e[i]);
+      }
+    } events{ev};
+    auto elapsed = [&](int a, int b) {
+      float ms = 0;
+      GE_CUDA(cudaEventElapsedTime(&ms, ev[a], ev[b]));
+      return (double)ms;
+    };
+    // A goes up once; its largest component and the hierarchy stay on the device
+    DeviceHierarchy h;
+    auto G = std::make_unique<DevGraph>();
+    upload_graph(ctx, *A, *G);
+    check_graph(ctx, *G);
+    DevBuf<int> kept;
+    if (largest_component) {
+      GE_CUDA(cudaEventRecord(ev[0], ctx->stream));
+      auto C = std::make_unique<DevGraph>();
+      st.components = largest_component_device(ctx, *G, *C, kept);
+      if (st.components > 1) G = std::move(C);
+      else unit_weights(ctx, *G);  // what ge_largest_component hands over: explicit weights
+      GE_CUDA(cudaEventRecord(ev[1], ctx->stream));
+    }
+    h.graphs.push_back(std::move(G));
+    GE_CUDA(cudaEventRecord(ev[2], ctx->stream));
+    coarsen_device(ctx, h, co, false, nullptr);
+    GE_CUDA(cudaEventRecord(ev[3], ctx->stream));
+    // down: every P_T and every level's row pointers (O(n)), and the coarsest graph in full
+    const int L = h.levels();
+    std::vector<HostHierarchy::Csr> hg(L + 1), hp(L);
+    for (int l = 0; l <= L; ++l) {
+      const DevGraph& D = *h.graphs[l];
+      HostHierarchy::Csr& g = hg[l];
+      g.rows = g.cols = D.n;
+      g.indptr.resize((size_t)D.n + 1);
+      D.I.download(ctx, g.indptr.data(), (size_t)D.n + 1);
+      if (l == L) {
+        g.indices.resize(std::max(D.nnz, 1));
+        D.J.download(ctx, g.indices.data(), D.nnz);
+        if (D.W.size()) {
+          g.data.resize(std::max(D.nnz, 1));
+          D.W.download(ctx, g.data.data(), D.nnz);
+        }
+      }
+      if (l < L) {
+        const DevAgg& P = *h.aggs[l];
+        HostHierarchy::Csr& p = hp[l];
+        p.rows = P.m;
+        p.cols = P.n;
+        p.indptr.resize((size_t)P.m + 1);
+        p.indices.resize(P.n);
+        P.ptr.download(ctx, p.indptr.data(), (size_t)P.m + 1);
+        P.idx.download(ctx, p.indices.data(), P.n);
+      }
+    }
+    const int n = h.graphs[0]->n;
+    if (vertices_out) {
+      if (st.components > 1) kept.download(ctx, vertices_out, (size_t)n);
+      else
+        for (int v = 0; v < n; ++v) vertices_out[v] = v;
+    }
+    GE_CUDA(cudaStreamSynchronize(ctx->stream));
+    if (largest_component) st.components_ms = elapsed(0, 1);
+    st.coarsen_ms = elapsed(2, 3);
+    std::vector<ge_csr> As(L + 1), Ps(std::max(L, 1));
+    for (int l = 0; l <= L; ++l) {
+      const HostHierarchy::Csr& g = hg[l];
+      ge_csr& c = As[l];
+      c.rows = c.cols = g.rows;
+      c.nnz = g.indptr[g.rows];
+      c.indptr = g.indptr.data();
+      c.indices = l == L ? g.indices.data() : nullptr;
+      c.data = l == L && !g.data.empty() ? g.data.data() : nullptr;
+    }
+    for (int l = 0; l < L; ++l) {
+      ge_csr& c = Ps[l];
+      c.rows = hp[l].rows;
+      c.cols = hp[l].cols;
+      c.nnz = hp[l].cols;
+      c.indptr = hp[l].indptr.data();
+      c.indices = hp[l].indices.data();
+      c.data = nullptr;
+    }
+    ge_embed_options eo;
+    if (eopt) eo = *eopt;
+    else ge_embed_options_default(&eo);
+    const double t_embed = now_ms();
+    // the level graphs now move into the driver's prefetched graphs
+    embed_levels(ctx, L, As.data(), Ps.data(), dim, &eo, coords_out, nullptr, nullptr, nullptr, &h);
+    st.embed_ms = now_ms() - t_embed;
+    *n_out = n;
+    st.levels = L;
+    st.total_ms = now_ms() - t0;
+    st.h2d_bytes = ctx->h2d_bytes - h0;
+    st.d2h_bytes = ctx->d2h_bytes - d0;
+    st.kernel_launches = ctx->launches - launches0;
+    if (stats) *stats = st;
   });
 }
 

@@ -332,18 +332,6 @@ __global__ void k_check_graph(const int* I, const int* J, int n, int* bad) {
     if (J[e] < 0 || J[e] >= n) *bad = 1;
 }
 
-struct DevGraph {
-  int n = 0, nnz = 0;
-  DevBuf<int> I, J;
-  DevBuf<double> W;  // empty: unit weights
-  const double* w() const { return W.size() ? W.get() : nullptr; }
-};
-
-struct DevAgg {
-  int m = 0, n = 0;
-  DevBuf<int> ptr, idx;
-};
-
 unsigned grid_of(int64_t n, int threads) { return (unsigned)std::max<int64_t>(1, (n + threads - 1) / threads); }
 
 class Coarsener {
@@ -481,52 +469,19 @@ class Coarsener {
     return true;
   }
 
-  void run(const ge_csr& A, const ge_coarsen_options& opt, HostHierarchy& out, ge_coarsen_stats* stats) {
-    const double t_begin = now_ms();
-    const int64_t launches0 = ctx_->launches;
-    const int n0 = A.rows;
-    const int nnz0 = A.indptr[n0];
-    auto S0 = std::make_unique<DevGraph>();
-    S0->n = n0;
-    S0->nnz = nnz0;
-    S0->I.alloc(ctx_, (size_t)n0 + 1);
-    S0->J.alloc(ctx_, std::max(nnz0, 1));
-    S0->I.upload(ctx_, A.indptr, (size_t)n0 + 1);
-    S0->J.upload(ctx_, A.indices, nnz0);
-    if (A.data != nullptr) {
-      S0->W.alloc(ctx_, std::max(nnz0, 1));
-      S0->W.upload(ctx_, A.data, nnz0);
-    }
+  // Levels of h.graphs[0] until min_coarse, max_levels or a level that merges nothing.
+  void build(DeviceHierarchy& h, const ge_coarsen_options& opt, bool check, int64_t* rounds_out) {
+    const DevGraph& S0 = *h.graphs[0];
+    const int n0 = S0.n;
     iota_.alloc(ctx_, std::max(n0, 1));
-    cudaEvent_t ev0, ev1;
-    GE_CUDA(cudaEventCreate(&ev0));
-    GE_CUDA(cudaEventCreate(&ev1));
-    struct Events {
-      cudaEvent_t a, b;
-      ~Events() {
-        cudaEventDestroy(a);
-        cudaEventDestroy(b);
-      }
-    } events{ev0, ev1};
-    GE_CUDA(cudaEventRecord(ev0, ctx_->stream));
-    {
-      DevBuf<int> bad(ctx_, 1);
-      bad.zero(ctx_->stream);
-      k_check_graph<<<grid_of(n0, 256), 256, 0, ctx_->stream>>>(S0->I.get(), S0->J.get(), n0, bad.get());
-      k_iota<<<grid_of(n0, 256), 256, 0, ctx_->stream>>>(iota_.get(), n0);
-      GE_CUDA(cudaGetLastError());
-      ctx_->launches += 2;
-      int bad_h = 0;
-      GE_CUDA(cudaMemcpyAsync(&bad_h, bad.get(), sizeof(int), cudaMemcpyDeviceToHost, ctx_->stream));
-      GE_CUDA(cudaStreamSynchronize(ctx_->stream));
-      GE_REQUIRE(!bad_h, "A.indptr is not ascending or A.indices has an entry outside [0, rows)");
-    }
-    std::vector<std::unique_ptr<DevGraph>> graphs;
-    std::vector<std::unique_ptr<DevAgg>> aggs;
+    if (check) check_graph(ctx_, S0);
+    k_iota<<<grid_of(n0, 256), 256, 0, ctx_->stream>>>(iota_.get(), n0);
+    GE_CUDA(cudaGetLastError());
+    ctx_->launches++;
     int64_t rounds = 0;
-    const DevGraph* level_graph = S0.get();
-    while (level_graph->n > opt.min_coarse && (int)aggs.size() < opt.max_levels) {
-      const int level = (int)aggs.size();
+    const DevGraph* level_graph = &S0;
+    while (level_graph->n > opt.min_coarse && h.levels() < opt.max_levels) {
+      const int level = h.levels();
       const int N = level_graph->n;
       const int target = std::max((int)std::floor(opt.coarsening_factor * (double)N), opt.min_coarse);
       DevBuf<int> agg(ctx_, std::max(N, 1));
@@ -554,16 +509,38 @@ class Coarsener {
       P->n = N;
       DevBuf<int> sorted;
       aggregation(agg.get(), N, M, P->ptr, P->idx, sorted);
-      aggs.push_back(std::move(P));
-      graphs.push_back(std::make_unique<DevGraph>(std::move(S)));
-      level_graph = graphs.back().get();
+      h.aggs.push_back(std::move(P));
+      h.graphs.push_back(std::make_unique<DevGraph>(std::move(S)));
+      level_graph = h.graphs.back().get();
     }
+    if (rounds_out) *rounds_out = rounds;
+  }
+
+  void run(const ge_csr& A, const ge_coarsen_options& opt, HostHierarchy& out, ge_coarsen_stats* stats) {
+    const double t_begin = now_ms();
+    const int64_t launches0 = ctx_->launches;
+    DeviceHierarchy h;
+    h.graphs.push_back(std::make_unique<DevGraph>());
+    upload_graph(ctx_, A, *h.graphs[0]);
+    cudaEvent_t ev0, ev1;
+    GE_CUDA(cudaEventCreate(&ev0));
+    GE_CUDA(cudaEventCreate(&ev1));
+    struct Events {
+      cudaEvent_t a, b;
+      ~Events() {
+        cudaEventDestroy(a);
+        cudaEventDestroy(b);
+      }
+    } events{ev0, ev1};
+    GE_CUDA(cudaEventRecord(ev0, ctx_->stream));
+    int64_t rounds = 0;
+    build(h, opt, true, &rounds);
     // one download of every level
-    const int L = (int)aggs.size();
+    const int L = h.levels();
     out.graphs.assign(L, HostHierarchy::Csr());
     out.aggs.assign(L, HostHierarchy::Csr());
     for (int l = 0; l < L; ++l) {
-      const DevGraph& G = *graphs[l];
+      const DevGraph& G = *h.graphs[l + 1];
       HostHierarchy::Csr& g = out.graphs[l];
       g.rows = g.cols = G.n;
       g.indptr.resize((size_t)G.n + 1);
@@ -572,7 +549,7 @@ class Coarsener {
       G.I.download(ctx_, g.indptr.data(), (size_t)G.n + 1);
       G.J.download(ctx_, g.indices.data(), G.nnz);
       G.W.download(ctx_, g.data.data(), G.nnz);
-      const DevAgg& P = *aggs[l];
+      const DevAgg& P = *h.aggs[l];
       HostHierarchy::Csr& p = out.aggs[l];
       p.rows = P.m;
       p.cols = P.n;
@@ -602,13 +579,52 @@ class Coarsener {
 
 }  // namespace
 
-void coarsen(ge_context* ctx, const ge_csr& A, const ge_coarsen_options& opt, HostHierarchy& out,
-             ge_coarsen_stats* stats) {
+void upload_graph(ge_context* ctx, const ge_csr& A, DevGraph& G) {
   GE_REQUIRE(A.rows == A.cols, "A must be square");
+  const int n = A.rows;
+  const int nnz = A.indptr[n];
+  G.n = n;
+  G.nnz = nnz;
+  G.I.alloc(ctx, (size_t)n + 1);
+  G.J.alloc(ctx, std::max(nnz, 1));
+  G.I.upload(ctx, A.indptr, (size_t)n + 1);
+  G.J.upload(ctx, A.indices, nnz);
+  if (A.data != nullptr) {
+    G.W.alloc(ctx, std::max(nnz, 1));
+    G.W.upload(ctx, A.data, nnz);
+  }
+}
+
+void check_graph(ge_context* ctx, const DevGraph& G) {
+  DevBuf<int> bad(ctx, 1);
+  bad.zero(ctx->stream);
+  k_check_graph<<<grid_of(G.n, 256), 256, 0, ctx->stream>>>(G.I.get(), G.J.get(), G.n, bad.get());
+  GE_CUDA(cudaGetLastError());
+  ctx->launches++;
+  int bad_h = 0;
+  GE_CUDA(cudaMemcpyAsync(&bad_h, bad.get(), sizeof(int), cudaMemcpyDeviceToHost, ctx->stream));
+  GE_CUDA(cudaStreamSynchronize(ctx->stream));
+  GE_REQUIRE(!bad_h, "A.indptr is not ascending or A.indices has an entry outside [0, rows)");
+}
+
+void check_coarsen_options(const ge_coarsen_options& opt) {
   GE_REQUIRE(opt.coarsening_factor > 0.0 && opt.coarsening_factor <= 1.0,
              "coarsening_factor must lie in (0, 1]");
   GE_REQUIRE(opt.min_coarse >= 1, "min_coarse must be >= 1");
   GE_REQUIRE(opt.max_levels >= 0, "max_levels must be >= 0");
+}
+
+void coarsen_device(ge_context* ctx, DeviceHierarchy& h, const ge_coarsen_options& opt, bool check,
+                    int64_t* rounds) {
+  check_coarsen_options(opt);
+  Coarsener c(ctx);
+  c.build(h, opt, check, rounds);
+}
+
+void coarsen(ge_context* ctx, const ge_csr& A, const ge_coarsen_options& opt, HostHierarchy& out,
+             ge_coarsen_stats* stats) {
+  GE_REQUIRE(A.rows == A.cols, "A must be square");
+  check_coarsen_options(opt);
   Coarsener c(ctx);
   c.run(A, opt, out, stats);
 }

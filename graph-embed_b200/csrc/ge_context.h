@@ -7,6 +7,7 @@
 #include <chrono>
 #include <cstddef>
 #include <cstdint>
+#include <memory>
 #include <vector>
 
 #include "ge_common.cuh"
@@ -246,6 +247,42 @@ struct HostHierarchy {
 };
 void coarsen(ge_context* ctx, const ge_csr& A, const ge_coarsen_options& opt, HostHierarchy& out,
              ge_coarsen_stats* stats);
+void check_coarsen_options(const ge_coarsen_options& opt);
+
+// A square CSR graph on the device.
+struct DevGraph {
+  int n = 0, nnz = 0;
+  DevBuf<int> I, J;
+  DevBuf<double> W;  // empty: unit weights
+  const double* w() const { return W.size() ? W.get() : nullptr; }
+};
+struct DevAgg {  // P_T of one level: m aggregates of n vertices, members ascending per row
+  int m = 0, n = 0;
+  DevBuf<int> ptr, idx;
+};
+// The levels of ge_coarsen left on the device: graphs[0] is the input, graphs[l] = As[l].
+struct DeviceHierarchy {
+  std::vector<std::unique_ptr<DevGraph>> graphs;
+  std::vector<std::unique_ptr<DevAgg>> aggs;
+  int levels() const { return (int)aggs.size(); }
+};
+// A on the device (square; the arrays as given, no check of the entries).
+void upload_graph(ge_context* ctx, const ge_csr& A, DevGraph& G);
+// GE_ERR_INVALID unless G.I is ascending and every column lies in [0, n).
+void check_graph(ge_context* ctx, const DevGraph& G);
+// Builds the hierarchy of the graph h.graphs[0] into h (check: run check_graph first).
+// rounds: matching rounds, all levels.
+void coarsen_device(ge_context* ctx, DeviceHierarchy& h, const ge_coarsen_options& opt, bool check,
+                    int64_t* rounds);
+
+// ---- ge_components.cu ------------------------------------------------------------------------
+// The largest weakly connected component of A (ties to the component with the smallest vertex) on
+// the device.  Returns the number of components.  With more than one, out receives the subgraph
+// A[vertices][:, vertices] (entry order kept, columns renumbered, weights copied; unit weights
+// become ones) and vertices its original ids, ascending; with one, out and vertices stay empty.
+int64_t largest_component_device(ge_context* ctx, const DevGraph& A, DevGraph& out, DevBuf<int>& vertices);
+// Unit weights made explicit: G.W = ones when it is empty.
+void unit_weights(ge_context* ctx, DevGraph& G);
 
 // ---- ge_multi.cu ---------------------------------------------------------------------------------
 void multi_attach(ge_context* ctx, int ndev, const int* devices);

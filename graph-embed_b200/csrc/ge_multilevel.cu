@@ -428,7 +428,9 @@ void multilevel_t(ge_context* ctx, const ge_csr& A, const ge_csr& P, const int32
   constexpr int NM = Real<T>::kMassArrays;
   const int n = A.rows, m = P.rows;
   const int nnz = A.indptr[n];
-  const bool weighted = p.use_weights && A.data != nullptr;
+  // a prepared graph carries its own weights (ge_layout_graph's levels are on the device only)
+  const bool has_weights = pre != nullptr ? pre->Dw.size() != 0 : A.data != nullptr;
+  const bool weighted = p.use_weights && has_weights;
 
   const bool verbose = std::getenv("GE_VERBOSE") != nullptr;
   double t_mark = now_ms();
@@ -477,7 +479,7 @@ void multilevel_t(ge_context* ctx, const ge_csr& A, const ge_csr& P, const int32
     GE_CUDA(cudaStreamWaitEvent(ctx->stream, pre->ready, 0));
     dI = pre->I.get();
     dJ = pre->J.get();
-    if (A.data != nullptr) dDw = pre->Dw.get();
+    if (has_weights) dDw = pre->Dw.get();
   } else {
     d_I.alloc(ctx, n + 1);
     d_J.alloc(ctx, std::max(nnz, 1));

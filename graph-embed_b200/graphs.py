@@ -51,9 +51,14 @@ def grid2d(nx, ny):
     return _finish(rows, cols, nx * ny)
 
 
-def rgg(n, avg_degree=10.0, dim=2, seed=12345):
+def _largest(A, largest):
+    return largest_component(A) if largest else A
+
+
+def rgg(n, avg_degree=10.0, dim=2, seed=12345, largest=True):
     """Random geometric graph on U[0,1]^dim, radius chosen for the requested average degree
-    (BASELINE config 2: n = 100 000, avg degree 10, d = 2); largest component."""
+    (BASELINE config 2: n = 100 000, avg degree 10, d = 2); largest component (largest=False: the
+    raw graph, every component)."""
     from scipy.spatial import cKDTree
     rng = np.random.default_rng(seed)
     pts = rng.random((n, dim))
@@ -62,12 +67,12 @@ def rgg(n, avg_degree=10.0, dim=2, seed=12345):
     else:
         r = (avg_degree / (4.0 / 3.0 * np.pi * n)) ** (1.0 / 3.0)
     pairs = cKDTree(pts).query_pairs(r, output_type="ndarray")
-    return largest_component(_finish(pairs[:, 0], pairs[:, 1], n))
+    return _largest(_finish(pairs[:, 0], pairs[:, 1], n), largest)
 
 
-def rmat(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345):
+def rmat(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345, largest=True):
     """R-MAT (BASELINE config 3: scale 20, edge factor 16); symmetrised, de-duplicated,
-    self-loops dropped, unit weights, largest component."""
+    self-loops dropped, unit weights, largest component (largest=False: the raw graph)."""
     rng = np.random.default_rng(seed)
     n = 1 << scale
     ne = edge_factor * n
@@ -80,18 +85,19 @@ def rmat(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345):
         cbit = ((u >= a) & (u < a + b)) | (u >= a + b + c)
         rows = (rows << 1) | rbit
         cols = (cols << 1) | cbit
-    return largest_component(_finish(rows, cols, n))
+    return _largest(_finish(rows, cols, n), largest)
 
 
-def delaunay3d(n, seed=12345):
-    """Edges of the Delaunay tetrahedralisation of n points in U[0,1]^3 (BASELINE config 5)."""
+def delaunay3d(n, seed=12345, largest=True):
+    """Edges of the Delaunay tetrahedralisation of n points in U[0,1]^3 (BASELINE config 5);
+    largest component (largest=False: the raw graph)."""
     from scipy.spatial import Delaunay
     rng = np.random.default_rng(seed)
     tets = Delaunay(rng.random((n, 3))).simplices
     pr = [(0, 1), (0, 2), (0, 3), (1, 2), (1, 3), (2, 3)]
     rows = np.concatenate([tets[:, i] for i, _ in pr])
     cols = np.concatenate([tets[:, j] for _, j in pr])
-    return largest_component(_finish(rows, cols, n))
+    return _largest(_finish(rows, cols, n), largest)
 
 
 def aggregation_matrix(agg, m):

@@ -84,17 +84,50 @@ int coarsen_then_embed(int nx, int dimension) {
   return coords.size() == static_cast<size_t>(nx) * nx ? 0 : 2;
 }
 
+// `--layout`: a grid with isolated vertices and a small second component appended, laid out in one
+// call (ge_b200::layout: largest component -> hierarchy -> embed, on the device).
+int layout_raw_graph(int nx, int dimension) {
+  ge_b200::options().seed = 3;
+  const int g = nx * nx, isolated = 50, tail = 10, n = g + isolated + tail;
+  const SparseMatrix G = grid(nx, nx);
+  linalgcpp::CooMatrix<double> coo(n, n);
+  for (int i = 0; i < G.Rows(); ++i)
+    for (int e = G.GetIndptr()[i]; e < G.GetIndptr()[i + 1]; ++e) coo.Add(i, G.GetIndices()[e], 1.0);
+  for (int v = g + isolated; v + 1 < n; ++v) {  // a path of `tail` vertices
+    coo.Add(v, v + 1, 1.0);
+    coo.Add(v + 1, v, 1.0);
+  }
+  const SparseMatrix A = coo.ToSparse();
+  std::vector<int> vertices;
+  ge_layout_stats stats;
+  linalgcpp::Timer timer(linalgcpp::Timer::Start::True);
+  std::vector<std::vector<double>> coords = ge_b200::layout(A, dimension, 0.25, 64, &vertices, &stats);
+  timer.Click();
+  std::cout << "layout: " << vertices.size() << " of " << n << " vertices kept (" << stats.components
+            << " components), " << stats.levels << " levels" << std::endl;
+  std::cout << "embedded! in time " << timer[0] << "s" << std::endl;
+  for (size_t i = 0; i < coords.size(); i++)
+    for (int k = 0; k < dimension; k++)
+      if (std::isnan(coords[i][k])) {
+        std::cerr << "NaN at vertex " << vertices[i] << std::endl;
+        return 1;
+      }
+  return coords.size() == static_cast<size_t>(g) && vertices.back() == g - 1 ? 0 : 2;
+}
+
 int main(int argc, char** argv) {
   std::string outdir;  // --out DIR: write the layout and the plot inputs like examples/embedder.cpp:230-289
-  bool coarsen = false;
+  bool coarsen = false, layout = false;
   for (int a = 1; a < argc; ++a) {
     if (a + 1 < argc && std::string(argv[a]) == "--gpus") return flat_on_gpus(std::atoi(argv[a + 1]), 2);
     if (a + 1 < argc && std::string(argv[a]) == "--out") outdir = argv[a + 1];
     if (std::string(argv[a]) == "--coarsen") coarsen = true;
+    if (std::string(argv[a]) == "--layout") layout = true;
   }
   int nx = argc > 1 ? std::atoi(argv[1]) : 64, ny = nx;
   const int dimension = argc > 2 ? std::atoi(argv[2]) : 2;
   if (coarsen) return coarsen_then_embed(nx, dimension);
+  if (layout) return layout_raw_graph(nx, dimension);
   std::vector<SparseMatrix> As = {grid(nx, ny)}, hierarchy;
   while (nx * ny > 40) {
     hierarchy.push_back(blocks(nx, ny));

@@ -134,6 +134,53 @@ inline std::vector<SparseMatrix> coarsen(const SparseMatrix& A, double coarsenin
   return P_Ts;
 }
 
+// examples/embedder.cpp:156 (largestComponent) on the device: the largest connected component of
+// A; vertices (when not null) receives the original id of each of its rows.
+inline SparseMatrix largestComponent(const SparseMatrix& A, std::vector<int>* vertices = nullptr) {
+  const ge_csr a = view(A);
+  const size_t n = static_cast<size_t>(A.Rows());
+  std::vector<int> vert(n), indptr(n + 1), indices(A.GetIndices().size());
+  std::vector<double> data(A.GetIndices().size());
+  int32_t k = 0;
+  int64_t nnz = 0;
+  check(ge_largest_component(default_context(), &a, vert.data(), &k, indptr.data(), indices.data(), data.data(),
+                             static_cast<int64_t>(indices.size()), &nnz, nullptr));
+  vert.resize(static_cast<size_t>(k));
+  indptr.resize(static_cast<size_t>(k) + 1);
+  indices.resize(static_cast<size_t>(nnz));
+  data.resize(static_cast<size_t>(nnz));
+  if (vertices) *vertices = vert;
+  return SparseMatrix(std::move(indptr), std::move(indices), std::move(data), k, k);
+}
+
+// A graph in, coordinates out: its largest component, the device-built hierarchy (ge_coarsen) and
+// partition::embed in one call (ge_layout_graph).  Row i of the result is the vertex (*vertices)[i]
+// of A; stats (when not null) receives the call's counters.
+inline std::vector<std::vector<double>> layout(const SparseMatrix& A, int d, double coarseningFactor,
+                                               int minCoarse, std::vector<int>* vertices = nullptr,
+                                               ge_layout_stats* stats = nullptr) {
+  const ge_csr a = view(A);
+  ge_coarsen_options copt;
+  ge_coarsen_options_default(&copt);
+  copt.coarsening_factor = coarseningFactor;
+  copt.min_coarse = minCoarse;
+  copt.seed = options().seed;
+  ge_embed_options eopt;
+  ge_embed_options_default(&eopt);
+  eopt.precision = options().precision;
+  eopt.seed = options().seed;
+  eopt.verbose = options().verbose;
+  const size_t n = static_cast<size_t>(A.Rows());
+  std::vector<double> x(n * static_cast<size_t>(d));
+  std::vector<int> vert(n);
+  int32_t k = 0;
+  check(ge_layout_graph(default_context(), &a, d, 1, &copt, &eopt, x.data(), vert.data(), &k, stats));
+  vert.resize(static_cast<size_t>(k));
+  if (vertices) *vertices = vert;
+  x.resize(static_cast<size_t>(k) * d);
+  return unflatten(x, k, d);
+}
+
 }  // namespace ge_b200
 
 #endif

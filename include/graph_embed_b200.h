@@ -253,6 +253,43 @@ ge_status ge_hierarchy_graph(const ge_hierarchy* h, int32_t l, ge_csr* out);
 ge_status ge_hierarchy_aggregation(const ge_hierarchy* h, int32_t l, ge_csr* out);
 void ge_hierarchy_destroy(ge_hierarchy* h);
 
+/* ---- raw graph -> coordinates on the device ----------------------------------------------------- */
+/* examples/embedder.cpp:156 (largestComponent, :35-93) on the device: the largest weakly connected
+ * component of A (every entry (i, j) links i and j), ties to the component with the smallest vertex.
+ * vertices: A->rows capacity, original ids of the kept vertices, ascending; the subgraph is
+ * A[vertices][:, vertices] with A's entry order (columns renumbered, so still ascending when A's
+ * were).  c_indptr: A->rows + 1 capacity.  Capacity rule as ge_galerkin (A->nnz suffices).
+ * c_data receives ones when A->data is NULL.  components (may be NULL): the number of components.
+ * On a multi-device context the call runs on the first device. */
+ge_status ge_largest_component(ge_context* ctx, const ge_csr* A, int32_t* vertices, int32_t* n_out,
+                               int32_t* c_indptr, int32_t* c_indices, double* c_data,
+                               int64_t capacity, int64_t* nnz_out, int64_t* components);
+
+typedef struct ge_layout_stats {
+  double total_ms;      /* whole call */
+  double components_ms; /* CUDA events around the component step; 0 when skipped */
+  double coarsen_ms;    /* CUDA events around the hierarchy build */
+  double embed_ms;      /* host clock: download of the O(n) arrays and the embed */
+  int64_t components;   /* components of A; 0 when the step is skipped */
+  int32_t levels;       /* L of the hierarchy */
+  double h2d_bytes, d2h_bytes;
+  int64_t kernel_launches;
+} ge_layout_stats;
+
+/* Graph -> coordinates: [largest component] -> ge_coarsen's hierarchy -> ge_embed, on the device.
+ * A is uploaded once and the coordinates come down once; of the hierarchy only every P_T, the row
+ * pointers of every level and the coarsest graph cross PCIe.  With eopt->seed != 0 the result equals
+ * ge_largest_component, then ge_coarsen, then ge_embed with the same options, bit for bit
+ * (largest_component = 0 skips the first step); so do the error statuses.
+ * copt / eopt NULL: defaults.  coords_out: A->rows x dim capacity, first *n_out rows written;
+ * vertices_out (A->rows capacity, may be NULL): original id of each written row.  stats may be NULL.
+ * On a multi-device context the component step and the coarsening run on the first device and the
+ * embed behaves as ge_embed does on that context. */
+ge_status ge_layout_graph(ge_context* ctx, const ge_csr* A, int dim, int32_t largest_component,
+                          const ge_coarsen_options* copt, const ge_embed_options* eopt,
+                          double* coords_out, int32_t* vertices_out, int32_t* n_out,
+                          ge_layout_stats* stats);
+
 /* The reference's random stream: count draws of uniform_real_distribution<double>(-1,1) over
  * std::mt19937(seed) (include/forceatlas.hpp:104-108). */
 void ge_reference_uniform(uint32_t seed, int64_t count, double* out);
