@@ -15,7 +15,7 @@ ROOT = os.path.dirname(PKG)
 CSRC = os.path.join(PKG, "csrc")
 LIBDIR = os.path.join(PKG, "lib")
 LIB = os.path.join(LIBDIR, "libgraphembed_b200.so")
-SOURCES = ["ge_capi.cu", "ge_flat.cu", "ge_flat_sym.cu", "ge_onchip.cu", "ge_multilevel.cu", "ge_galerkin.cu", "ge_coarsen.cu", "ge_components.cu", "ge_radii.cu", "ge_multi.cu"]
+SOURCES = ["ge_capi.cu", "ge_flat.cu", "ge_flat_sym.cu", "ge_onchip.cu", "ge_multilevel.cu", "ge_galerkin.cu", "ge_coarsen.cu", "ge_components.cu", "ge_edges.cu", "ge_radii.cu", "ge_multi.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "-O3", "-std=c++17",
               "-Xcompiler", "-fPIC,-O2,-Wall,-Wno-unknown-pragmas", "--expt-relaxed-constexpr"]
 

@@ -76,6 +76,7 @@ SYMBOLS = [
     "ge_flat_symmetric_pass_share", "ge_embed_aggregate_ranges", "ge_embed_aggregate_owners",
     "ge_coarsen_options_default", "ge_coarsen", "ge_hierarchy_levels", "ge_hierarchy_graph",
     "ge_hierarchy_aggregation", "ge_hierarchy_destroy", "ge_largest_component", "ge_layout_graph",
+    "ge_edges_options_default", "ge_graph_from_edges", "ge_layout_edges",
 ]
 
 _lib = None
@@ -145,6 +146,53 @@ class LayoutStats(C.Structure):
     _fields_ = [("total_ms", C.c_double), ("components_ms", C.c_double), ("coarsen_ms", C.c_double),
                 ("embed_ms", C.c_double), ("components", C.c_int64), ("levels", C.c_int32),
                 ("h2d_bytes", C.c_double), ("d2h_bytes", C.c_double), ("kernel_launches", C.c_int64)]
+
+
+class EdgesOptions(C.Structure):
+    _fields_ = [("symmetrize", C.c_int32), ("keep_self_loops", C.c_int32), ("unit_weights", C.c_int32)]
+
+
+class EdgesStats(C.Structure):
+    _fields_ = [("total_ms", C.c_double), ("device_ms", C.c_double), ("nnz", C.c_int64),
+                ("self_loops_dropped", C.c_int64), ("duplicates_merged", C.c_int64),
+                ("kernel_launches", C.c_int64)]
+
+
+def _struct_dict(st):
+    return {f: getattr(st, f) for f, _ in st._fields_}
+
+
+class EdgeList:
+    """int32 id arrays (and float64 weights) of an edge list, checked to fit the C ABI's int32 ids."""
+
+    def __init__(self, n, src, dst, weights=None):
+        src, dst = np.asarray(src).ravel(), np.asarray(dst).ravel()
+        if src.shape != dst.shape:
+            raise ValueError("src and dst differ in length")
+        if src.size and not (np.issubdtype(src.dtype, np.integer) and np.issubdtype(dst.dtype, np.integer)):
+            raise ValueError("vertex ids must be integers")
+        lo, hi = np.iinfo(np.int32).min, np.iinfo(np.int32).max
+        if not lo <= int(n) <= hi:
+            raise GeError(GE_ERR_INVALID, "n does not fit int32")
+        for a in (src, dst):  # ids of a wider type must fit int32 before they are narrowed
+            if a.size and a.dtype != np.int32 and (int(a.min()) < lo or int(a.max()) > hi):
+                raise GeError(GE_ERR_INVALID, "a vertex id does not fit int32")
+        self.n, self.E = int(n), int(src.size)
+        self.src, self.dst = _i32(src), _i32(dst)
+        self.w = None if weights is None else _f64(np.asarray(weights).ravel())
+        if self.w is not None and self.w.size != self.E:
+            raise ValueError("weights differ in length from the edges")
+
+    def args(self):
+        return (C.c_int32(self.n), C.c_int64(self.E), _ptr(self.src, _pi), _ptr(self.dst, _pi), _ptr(self.w, _pd))
+
+
+def edges_options(symmetrize=True, keep_self_loops=False, unit_weights=False):
+    o = EdgesOptions()
+    lib().ge_edges_options_default(C.byref(o))
+    o.symmetrize, o.keep_self_loops, o.unit_weights = int(bool(symmetrize)), int(bool(keep_self_loops)), \
+        int(bool(unit_weights))
+    return o
 
 
 def _csr_copy(c, with_data=True):
@@ -406,13 +454,9 @@ class Context:
         B = sp.csr_matrix((val[:e].copy(), idx[:e].copy(), ptr[:k + 1].copy()), shape=(k, k))
         return B, vert[:k].copy(), int(comps.value)
 
-    def layout(self, A, dim, coarsening_factor=0.25, min_coarse=64, max_levels=32, coarsen_seed=0, seed=0,
-               largest_component=True, precision=GE_F64, coarse_iterations=100000, level_iterations=100,
-               verbose=False):
-        """ge_layout_graph: [largest component] -> ge_coarsen -> ge_embed in one call ->
-        (coords [n x dim], vertices [n] original ids of the rows, stats)."""
-        import scipy.sparse as sp
-        a = CsrView(sp.csr_matrix(A))
+    @staticmethod
+    def _layout_options(coarsening_factor, min_coarse, max_levels, coarsen_seed, seed, precision,
+                        coarse_iterations, level_iterations, verbose):
         copt = CoarsenOptions()
         lib().ge_coarsen_options_default(C.byref(copt))
         copt.coarsening_factor, copt.min_coarse = float(coarsening_factor), int(min_coarse)
@@ -421,6 +465,17 @@ class Context:
         lib().ge_embed_options_default(C.byref(eopt))
         eopt.seed, eopt.precision, eopt.verbose = int(seed), int(precision), int(verbose)
         eopt.coarse_iterations, eopt.level_iterations = int(coarse_iterations), int(level_iterations)
+        return copt, eopt
+
+    def layout(self, A, dim, coarsening_factor=0.25, min_coarse=64, max_levels=32, coarsen_seed=0, seed=0,
+               largest_component=True, precision=GE_F64, coarse_iterations=100000, level_iterations=100,
+               verbose=False):
+        """ge_layout_graph: [largest component] -> ge_coarsen -> ge_embed in one call ->
+        (coords [n x dim], vertices [n] original ids of the rows, stats)."""
+        import scipy.sparse as sp
+        a = CsrView(sp.csr_matrix(A))
+        copt, eopt = self._layout_options(coarsening_factor, min_coarse, max_levels, coarsen_seed, seed, precision,
+                                          coarse_iterations, level_iterations, verbose)
         n = A.shape[0]
         out = np.zeros((max(n, 1), dim))
         vert = np.zeros(max(n, 1), dtype=np.int32)
@@ -430,7 +485,45 @@ class Context:
                                      C.byref(eopt), _ptr(out, _pd), _ptr(vert, _pi), C.byref(n_out),
                                      C.byref(st)))
         k = int(n_out.value)
-        return out[:k].copy(), vert[:k].copy(), {f: getattr(st, f) for f, _ in st._fields_}
+        return out[:k].copy(), vert[:k].copy(), _struct_dict(st)
+
+    def graph_from_edges(self, n, src, dst, weights=None, symmetrize=True, keep_self_loops=False,
+                         unit_weights=False):
+        """ge_graph_from_edges: the CSR CooMatrix builds from the edges src[e] -> dst[e] (weights None:
+        1.0) -> (scipy CSR n x n, stats)."""
+        import scipy.sparse as sp
+        el = EdgeList(n, src, dst, weights)
+        opt = edges_options(symmetrize, keep_self_loops, unit_weights)
+        cap = max(el.E * (2 if symmetrize else 1), 1)
+        ptr = np.zeros(el.n + 1, dtype=np.int32)
+        idx = np.empty(cap, dtype=np.int32)
+        val = np.empty(cap)
+        nnz = C.c_int64()
+        st = EdgesStats()
+        _check(lib().ge_graph_from_edges(self.h, *el.args(), C.byref(opt), _ptr(ptr, _pi), _ptr(idx, _pi),
+                                         _ptr(val, _pd), C.c_int64(cap), C.byref(nnz), C.byref(st)))
+        k = int(nnz.value)
+        return sp.csr_matrix((val[:k], idx[:k], ptr), shape=(el.n, el.n)), _struct_dict(st)
+
+    def layout_edges(self, n, src, dst, dim, weights=None, symmetrize=True, keep_self_loops=False,
+                     unit_weights=False, coarsening_factor=0.25, min_coarse=64, max_levels=32, coarsen_seed=0,
+                     seed=0, largest_component=True, precision=GE_F64, coarse_iterations=100000,
+                     level_iterations=100, verbose=False):
+        """ge_layout_edges: edge list -> graph -> [largest component] -> ge_coarsen -> ge_embed in one
+        call -> (coords [k x dim], vertices [k] original ids of the rows, edges stats, layout stats)."""
+        el = EdgeList(n, src, dst, weights)
+        xopt = edges_options(symmetrize, keep_self_loops, unit_weights)
+        copt, eopt = self._layout_options(coarsening_factor, min_coarse, max_levels, coarsen_seed, seed, precision,
+                                          coarse_iterations, level_iterations, verbose)
+        out = np.zeros((max(el.n, 1), dim))
+        vert = np.zeros(max(el.n, 1), dtype=np.int32)
+        n_out = C.c_int32()
+        xs, st = EdgesStats(), LayoutStats()
+        _check(lib().ge_layout_edges(self.h, *el.args(), C.byref(xopt), int(dim), int(bool(largest_component)),
+                                     C.byref(copt), C.byref(eopt), _ptr(out, _pd), _ptr(vert, _pi),
+                                     C.byref(n_out), C.byref(xs), C.byref(st)))
+        k = int(n_out.value)
+        return out[:k].copy(), vert[:k].copy(), _struct_dict(xs), _struct_dict(st)
 
     def flat_plan(self, A, dim, params, rows=None, symmetric=None):
         """rows=(r0, r1): ordered row-block plan; symmetric=(rank, world): that rank's plan of a

@@ -961,6 +961,105 @@ void require_ctx(ge_context* ctx) {
   GE_CUDA(cudaSetDevice(ctx->device));
 }
 
+// The body of ge_layout_graph and ge_layout_edges: a checked graph on the device -> [largest
+// component] -> ge_coarsen's hierarchy -> ge_embed.  Fills st but for the whole-call counters.
+void layout_device(ge_context* ctx, std::unique_ptr<DevGraph> G, int dim, int32_t largest_component,
+                   const ge_coarsen_options& co, const ge_embed_options* eopt, double* coords_out,
+                   int32_t* vertices_out, int32_t* n_out, ge_layout_stats& st) {
+  cudaEvent_t ev[4];
+  for (auto& e : ev) GE_CUDA(cudaEventCreate(&e));
+  struct Events {
+    cudaEvent_t* e;
+    ~Events() {
+      for (int i = 0; i < 4; ++i) cudaEventDestroy(e[i]);
+    }
+  } events{ev};
+  auto elapsed = [&](int a, int b) {
+    float ms = 0;
+    GE_CUDA(cudaEventElapsedTime(&ms, ev[a], ev[b]));
+    return (double)ms;
+  };
+  DeviceHierarchy h;
+  DevBuf<int> kept;
+  if (largest_component) {
+    GE_CUDA(cudaEventRecord(ev[0], ctx->stream));
+    auto C = std::make_unique<DevGraph>();
+    st.components = largest_component_device(ctx, *G, *C, kept);
+    if (st.components > 1) G = std::move(C);
+    else unit_weights(ctx, *G);  // what ge_largest_component hands over: explicit weights
+    GE_CUDA(cudaEventRecord(ev[1], ctx->stream));
+  }
+  h.graphs.push_back(std::move(G));
+  GE_CUDA(cudaEventRecord(ev[2], ctx->stream));
+  coarsen_device(ctx, h, co, false, nullptr);
+  GE_CUDA(cudaEventRecord(ev[3], ctx->stream));
+  // down: every P_T and every level's row pointers (O(n)), and the coarsest graph in full
+  const int L = h.levels();
+  std::vector<HostHierarchy::Csr> hg(L + 1), hp(L);
+  for (int l = 0; l <= L; ++l) {
+    const DevGraph& D = *h.graphs[l];
+    HostHierarchy::Csr& g = hg[l];
+    g.rows = g.cols = D.n;
+    g.indptr.resize((size_t)D.n + 1);
+    D.I.download(ctx, g.indptr.data(), (size_t)D.n + 1);
+    if (l == L) {
+      g.indices.resize(std::max(D.nnz, 1));
+      D.J.download(ctx, g.indices.data(), D.nnz);
+      if (D.W.size()) {
+        g.data.resize(std::max(D.nnz, 1));
+        D.W.download(ctx, g.data.data(), D.nnz);
+      }
+    }
+    if (l < L) {
+      const DevAgg& P = *h.aggs[l];
+      HostHierarchy::Csr& p = hp[l];
+      p.rows = P.m;
+      p.cols = P.n;
+      p.indptr.resize((size_t)P.m + 1);
+      p.indices.resize(P.n);
+      P.ptr.download(ctx, p.indptr.data(), (size_t)P.m + 1);
+      P.idx.download(ctx, p.indices.data(), P.n);
+    }
+  }
+  const int n = h.graphs[0]->n;
+  if (vertices_out) {
+    if (st.components > 1) kept.download(ctx, vertices_out, (size_t)n);
+    else
+      for (int v = 0; v < n; ++v) vertices_out[v] = v;
+  }
+  GE_CUDA(cudaStreamSynchronize(ctx->stream));
+  if (largest_component) st.components_ms = elapsed(0, 1);
+  st.coarsen_ms = elapsed(2, 3);
+  std::vector<ge_csr> As(L + 1), Ps(std::max(L, 1));
+  for (int l = 0; l <= L; ++l) {
+    const HostHierarchy::Csr& g = hg[l];
+    ge_csr& c = As[l];
+    c.rows = c.cols = g.rows;
+    c.nnz = g.indptr[g.rows];
+    c.indptr = g.indptr.data();
+    c.indices = l == L ? g.indices.data() : nullptr;
+    c.data = l == L && !g.data.empty() ? g.data.data() : nullptr;
+  }
+  for (int l = 0; l < L; ++l) {
+    ge_csr& c = Ps[l];
+    c.rows = hp[l].rows;
+    c.cols = hp[l].cols;
+    c.nnz = hp[l].cols;
+    c.indptr = hp[l].indptr.data();
+    c.indices = hp[l].indices.data();
+    c.data = nullptr;
+  }
+  ge_embed_options eo;
+  if (eopt) eo = *eopt;
+  else ge_embed_options_default(&eo);
+  const double t_embed = now_ms();
+  // the level graphs now move into the driver's prefetched graphs
+  embed_levels(ctx, L, As.data(), Ps.data(), dim, &eo, coords_out, nullptr, nullptr, nullptr, &h);
+  st.embed_ms = now_ms() - t_embed;
+  *n_out = n;
+  st.levels = L;
+}
+
 }  // namespace
 }  // namespace ge
 
@@ -1351,107 +1450,92 @@ ge_status ge_layout_graph(ge_context* ctx, const ge_csr* A, int dim, int32_t lar
     const double t0 = now_ms();
     const int64_t launches0 = ctx->launches;
     const double h0 = ctx->h2d_bytes, d0 = ctx->d2h_bytes;
-    cudaEvent_t ev[4];
-    for (auto& e : ev) GE_CUDA(cudaEventCreate(&e));
-    struct Events {
-      cudaEvent_t* e;
-      ~Events() {
-        for (int i = 0; i < 4; ++i) cudaEventDestroy(e[i]);
-      }
-    } events{ev};
-    auto elapsed = [&](int a, int b) {
-      float ms = 0;
-      GE_CUDA(cudaEventElapsedTime(&ms, ev[a], ev[b]));
-      return (double)ms;
-    };
     // A goes up once; its largest component and the hierarchy stay on the device
-    DeviceHierarchy h;
     auto G = std::make_unique<DevGraph>();
     upload_graph(ctx, *A, *G);
     check_graph(ctx, *G);
-    DevBuf<int> kept;
-    if (largest_component) {
-      GE_CUDA(cudaEventRecord(ev[0], ctx->stream));
-      auto C = std::make_unique<DevGraph>();
-      st.components = largest_component_device(ctx, *G, *C, kept);
-      if (st.components > 1) G = std::move(C);
-      else unit_weights(ctx, *G);  // what ge_largest_component hands over: explicit weights
-      GE_CUDA(cudaEventRecord(ev[1], ctx->stream));
-    }
-    h.graphs.push_back(std::move(G));
-    GE_CUDA(cudaEventRecord(ev[2], ctx->stream));
-    coarsen_device(ctx, h, co, false, nullptr);
-    GE_CUDA(cudaEventRecord(ev[3], ctx->stream));
-    // down: every P_T and every level's row pointers (O(n)), and the coarsest graph in full
-    const int L = h.levels();
-    std::vector<HostHierarchy::Csr> hg(L + 1), hp(L);
-    for (int l = 0; l <= L; ++l) {
-      const DevGraph& D = *h.graphs[l];
-      HostHierarchy::Csr& g = hg[l];
-      g.rows = g.cols = D.n;
-      g.indptr.resize((size_t)D.n + 1);
-      D.I.download(ctx, g.indptr.data(), (size_t)D.n + 1);
-      if (l == L) {
-        g.indices.resize(std::max(D.nnz, 1));
-        D.J.download(ctx, g.indices.data(), D.nnz);
-        if (D.W.size()) {
-          g.data.resize(std::max(D.nnz, 1));
-          D.W.download(ctx, g.data.data(), D.nnz);
-        }
-      }
-      if (l < L) {
-        const DevAgg& P = *h.aggs[l];
-        HostHierarchy::Csr& p = hp[l];
-        p.rows = P.m;
-        p.cols = P.n;
-        p.indptr.resize((size_t)P.m + 1);
-        p.indices.resize(P.n);
-        P.ptr.download(ctx, p.indptr.data(), (size_t)P.m + 1);
-        P.idx.download(ctx, p.indices.data(), P.n);
-      }
-    }
-    const int n = h.graphs[0]->n;
-    if (vertices_out) {
-      if (st.components > 1) kept.download(ctx, vertices_out, (size_t)n);
-      else
-        for (int v = 0; v < n; ++v) vertices_out[v] = v;
-    }
-    GE_CUDA(cudaStreamSynchronize(ctx->stream));
-    if (largest_component) st.components_ms = elapsed(0, 1);
-    st.coarsen_ms = elapsed(2, 3);
-    std::vector<ge_csr> As(L + 1), Ps(std::max(L, 1));
-    for (int l = 0; l <= L; ++l) {
-      const HostHierarchy::Csr& g = hg[l];
-      ge_csr& c = As[l];
-      c.rows = c.cols = g.rows;
-      c.nnz = g.indptr[g.rows];
-      c.indptr = g.indptr.data();
-      c.indices = l == L ? g.indices.data() : nullptr;
-      c.data = l == L && !g.data.empty() ? g.data.data() : nullptr;
-    }
-    for (int l = 0; l < L; ++l) {
-      ge_csr& c = Ps[l];
-      c.rows = hp[l].rows;
-      c.cols = hp[l].cols;
-      c.nnz = hp[l].cols;
-      c.indptr = hp[l].indptr.data();
-      c.indices = hp[l].indices.data();
-      c.data = nullptr;
-    }
-    ge_embed_options eo;
-    if (eopt) eo = *eopt;
-    else ge_embed_options_default(&eo);
-    const double t_embed = now_ms();
-    // the level graphs now move into the driver's prefetched graphs
-    embed_levels(ctx, L, As.data(), Ps.data(), dim, &eo, coords_out, nullptr, nullptr, nullptr, &h);
-    st.embed_ms = now_ms() - t_embed;
-    *n_out = n;
-    st.levels = L;
+    layout_device(ctx, std::move(G), dim, largest_component, co, eopt, coords_out, vertices_out, n_out, st);
     st.total_ms = now_ms() - t0;
     st.h2d_bytes = ctx->h2d_bytes - h0;
     st.d2h_bytes = ctx->d2h_bytes - d0;
     st.kernel_launches = ctx->launches - launches0;
     if (stats) *stats = st;
+  });
+}
+
+void ge_edges_options_default(ge_edges_options* opt) {
+  std::memset(opt, 0, sizeof(*opt));
+  opt->symmetrize = 1;
+  opt->keep_self_loops = 0;
+  opt->unit_weights = 0;
+}
+
+ge_status ge_graph_from_edges(ge_context* ctx, int32_t n, int64_t E, const int32_t* src, const int32_t* dst,
+                              const double* w, const ge_edges_options* opt, int32_t* c_indptr,
+                              int32_t* c_indices, double* c_data, int64_t capacity, int64_t* nnz_out,
+                              ge_edges_stats* stats) {
+  return guarded([&] {
+    require_device();
+    require_ctx(ctx);  // a multi-device context: its first device
+    ge_edges_options eo;
+    if (opt) eo = *opt;
+    else ge_edges_options_default(&eo);
+    check_edges_args(n, E, src, dst, eo);
+    GE_REQUIRE(c_indptr && nnz_out, "null argument");
+    const double t0 = now_ms();
+    ge_edges_stats st;
+    std::memset(&st, 0, sizeof(st));
+    DevGraph G;
+    edges_to_graph_device(ctx, n, E, src, dst, w, eo, G, &st);
+    *nnz_out = G.nnz;
+    G.I.download(ctx, c_indptr, (size_t)n + 1);
+    if (G.nnz <= capacity) {
+      GE_REQUIRE(G.nnz == 0 || (c_indices && c_data), "c_indices / c_data are null");
+      G.J.download(ctx, c_indices, (size_t)G.nnz);
+      G.W.download(ctx, c_data, (size_t)G.nnz);
+    }
+    GE_CUDA(cudaStreamSynchronize(ctx->stream));
+    st.total_ms = now_ms() - t0;
+    if (stats) *stats = st;
+    GE_REQUIRE(G.nnz <= capacity, "output capacity too small (see *nnz_out)");
+  });
+}
+
+ge_status ge_layout_edges(ge_context* ctx, int32_t n, int64_t E, const int32_t* src, const int32_t* dst,
+                          const double* w, const ge_edges_options* edges_opt, int dim,
+                          int32_t largest_component, const ge_coarsen_options* copt,
+                          const ge_embed_options* eopt, double* coords_out, int32_t* vertices_out,
+                          int32_t* n_out, ge_edges_stats* edges_stats, ge_layout_stats* layout_stats) {
+  return guarded([&] {
+    require_device();
+    require_ctx(ctx);
+    ge_edges_options xo;
+    if (edges_opt) xo = *edges_opt;
+    else ge_edges_options_default(&xo);
+    check_edges_args(n, E, src, dst, xo);
+    GE_REQUIRE(coords_out && n_out, "null argument");
+    ge_coarsen_options co;
+    if (copt) co = *copt;
+    else ge_coarsen_options_default(&co);
+    check_coarsen_options(co);
+    ge_layout_stats st;
+    std::memset(&st, 0, sizeof(st));
+    ge_edges_stats xs;
+    std::memset(&xs, 0, sizeof(xs));
+    const double t0 = now_ms();
+    const int64_t launches0 = ctx->launches;
+    const double h0 = ctx->h2d_bytes, d0 = ctx->d2h_bytes;
+    // the edges go up once; the graph built from them never leaves the device
+    auto G = std::make_unique<DevGraph>();
+    edges_to_graph_device(ctx, n, E, src, dst, w, xo, *G, &xs);
+    xs.total_ms = now_ms() - t0;
+    layout_device(ctx, std::move(G), dim, largest_component, co, eopt, coords_out, vertices_out, n_out, st);
+    st.total_ms = now_ms() - t0;
+    st.h2d_bytes = ctx->h2d_bytes - h0;
+    st.d2h_bytes = ctx->d2h_bytes - d0;
+    st.kernel_launches = ctx->launches - launches0;
+    if (edges_stats) *edges_stats = xs;
+    if (layout_stats) *layout_stats = st;
   });
 }
 

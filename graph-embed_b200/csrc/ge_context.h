@@ -284,6 +284,14 @@ int64_t largest_component_device(ge_context* ctx, const DevGraph& A, DevGraph& o
 // Unit weights made explicit: G.W = ones when it is empty.
 void unit_weights(ge_context* ctx, DevGraph& G);
 
+// ---- ge_edges.cu -----------------------------------------------------------------------------
+// GE_ERR_INVALID unless n and E are in range and the slots of E edges fit int32 row pointers.
+void check_edges_args(int64_t n, int64_t E, const int32_t* src, const int32_t* dst, const ge_edges_options& opt);
+// The graph of ge_graph_from_edges (include/graph_embed_b200.h) built on the device from host edge
+// arrays (uploaded here).  out.W is always explicit.  stats: every field but total_ms.
+void edges_to_graph_device(ge_context* ctx, int n, int64_t E, const int32_t* src, const int32_t* dst,
+                           const double* w, const ge_edges_options& opt, DevGraph& out, ge_edges_stats* stats);
+
 // ---- ge_multi.cu ---------------------------------------------------------------------------------
 void multi_attach(ge_context* ctx, int ndev, const int* devices);
 void multi_destroy(MultiState* m);

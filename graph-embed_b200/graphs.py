@@ -55,10 +55,9 @@ def _largest(A, largest):
     return largest_component(A) if largest else A
 
 
-def rgg(n, avg_degree=10.0, dim=2, seed=12345, largest=True):
-    """Random geometric graph on U[0,1]^dim, radius chosen for the requested average degree
-    (BASELINE config 2: n = 100 000, avg degree 10, d = 2); largest component (largest=False: the
-    raw graph, every component)."""
+def rgg_edges(n, avg_degree=10.0, dim=2, seed=12345):
+    """The pairs (rows, cols, n) of a random geometric graph on U[0,1]^dim, each unordered pair once,
+    radius chosen for the requested average degree."""
     from scipy.spatial import cKDTree
     rng = np.random.default_rng(seed)
     pts = rng.random((n, dim))
@@ -67,12 +66,19 @@ def rgg(n, avg_degree=10.0, dim=2, seed=12345, largest=True):
     else:
         r = (avg_degree / (4.0 / 3.0 * np.pi * n)) ** (1.0 / 3.0)
     pairs = cKDTree(pts).query_pairs(r, output_type="ndarray")
-    return _largest(_finish(pairs[:, 0], pairs[:, 1], n), largest)
+    return pairs[:, 0], pairs[:, 1], n
 
 
-def rmat(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345, largest=True):
-    """R-MAT (BASELINE config 3: scale 20, edge factor 16); symmetrised, de-duplicated,
-    self-loops dropped, unit weights, largest component (largest=False: the raw graph)."""
+def rgg(n, avg_degree=10.0, dim=2, seed=12345, largest=True):
+    """Random geometric graph on U[0,1]^dim, radius chosen for the requested average degree
+    (BASELINE config 2: n = 100 000, avg degree 10, d = 2); largest component (largest=False: the
+    raw graph, every component)."""
+    return _largest(_finish(*rgg_edges(n, avg_degree, dim, seed)), largest)
+
+
+def rmat_edges(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345):
+    """The raw R-MAT edges (rows, cols, n): edge_factor * 2^scale pairs, duplicates and self-loops
+    included."""
     rng = np.random.default_rng(seed)
     n = 1 << scale
     ne = edge_factor * n
@@ -85,19 +91,31 @@ def rmat(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345, largest=True
         cbit = ((u >= a) & (u < a + b)) | (u >= a + b + c)
         rows = (rows << 1) | rbit
         cols = (cols << 1) | cbit
-    return _largest(_finish(rows, cols, n), largest)
+    return rows, cols, n
 
 
-def delaunay3d(n, seed=12345, largest=True):
-    """Edges of the Delaunay tetrahedralisation of n points in U[0,1]^3 (BASELINE config 5);
-    largest component (largest=False: the raw graph)."""
+def rmat(scale, edge_factor=16, abc=(0.57, 0.19, 0.19), seed=12345, largest=True):
+    """R-MAT (BASELINE config 3: scale 20, edge factor 16); symmetrised, de-duplicated,
+    self-loops dropped, unit weights, largest component (largest=False: the raw graph)."""
+    return _largest(_finish(*rmat_edges(scale, edge_factor, abc, seed)), largest)
+
+
+def delaunay3d_edges(n, seed=12345):
+    """The edges (rows, cols, n) of the Delaunay tetrahedralisation of n points in U[0,1]^3: six per
+    tetrahedron, so an edge shared by k tetrahedra appears k times."""
     from scipy.spatial import Delaunay
     rng = np.random.default_rng(seed)
     tets = Delaunay(rng.random((n, 3))).simplices
     pr = [(0, 1), (0, 2), (0, 3), (1, 2), (1, 3), (2, 3)]
     rows = np.concatenate([tets[:, i] for i, _ in pr])
     cols = np.concatenate([tets[:, j] for _, j in pr])
-    return _largest(_finish(rows, cols, n), largest)
+    return rows, cols, n
+
+
+def delaunay3d(n, seed=12345, largest=True):
+    """Edges of the Delaunay tetrahedralisation of n points in U[0,1]^3 (BASELINE config 5);
+    largest component (largest=False: the raw graph)."""
+    return _largest(_finish(*delaunay3d_edges(n, seed)), largest)
 
 
 def aggregation_matrix(agg, m):

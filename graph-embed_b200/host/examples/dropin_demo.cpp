@@ -5,6 +5,7 @@
 #include <cassert>
 #include <cmath>
 #include <cstdlib>
+#include <cstring>
 #include <iostream>
 #include <string>
 
@@ -115,19 +116,83 @@ int layout_raw_graph(int nx, int dimension) {
   return coords.size() == static_cast<size_t>(g) && vertices.back() == g - 1 ? 0 : 2;
 }
 
+// `--edges`: a grid's edge list with every edge listed twice (once reversed), self-loops and real
+// weights.  ge_b200::fromEdges must equal linalgcpp's CooMatrix built from the same calls, bit for
+// bit; then the edge list is laid out in one call (ge_b200::layoutEdges).
+int layout_edge_list(int nx, int dimension) {
+  ge_b200::options().seed = 3;
+  const int n = nx * nx;
+  std::vector<int> src, dst;
+  std::vector<double> w;
+  auto edge = [&](int a, int b, double x) {
+    src.push_back(a);
+    dst.push_back(b);
+    w.push_back(x);
+  };
+  for (int x = 0; x < nx; ++x)
+    for (int y = 0; y < nx; ++y) {
+      const int v = x * nx + y;
+      // weights that round differently depending on the order they are added in
+      if (x + 1 < nx) {
+        edge(v, v + nx, 1.0 + v * 1e-3);
+        edge(v + nx, v, 1e-17 * (y + 1));
+      }
+      if (y + 1 < nx) {
+        edge(v, v + 1, 0.1 * (x + 1));
+        edge(v + 1, v, 0.7);
+      }
+      if (v % 7 == 0) edge(v, v, 2.0);
+    }
+  ge_edges_options opt;
+  ge_edges_options_default(&opt);
+  linalgcpp::CooMatrix<double> coo(n, n);
+  for (size_t e = 0; e < src.size(); ++e) {
+    if (src[e] == dst[e]) continue;
+    coo.Add(src[e], dst[e], w[e]);
+    coo.Add(dst[e], src[e], w[e]);
+  }
+  const SparseMatrix ref = coo.ToSparse();
+  const SparseMatrix A = ge_b200::fromEdges(n, src, dst, &w, &opt);
+  if (A.GetIndptr() != ref.GetIndptr() || A.GetIndices() != ref.GetIndices() ||
+      A.GetData().size() != ref.GetData().size() ||
+      std::memcmp(A.GetData().data(), ref.GetData().data(), sizeof(double) * ref.GetData().size()) != 0) {
+    std::cerr << "fromEdges differs from CooMatrix::ToSparse()" << std::endl;
+    return 3;
+  }
+  std::cout << "fromEdges: " << src.size() << " edges -> " << A.GetIndices().size()
+            << " entries, equal to CooMatrix" << std::endl;
+  std::vector<int> vertices;
+  ge_layout_stats stats;
+  linalgcpp::Timer timer(linalgcpp::Timer::Start::True);
+  std::vector<std::vector<double>> coords =
+      ge_b200::layoutEdges(n, src, dst, &w, dimension, 0.25, 64, &vertices, &opt, &stats);
+  timer.Click();
+  std::cout << "layoutEdges: " << vertices.size() << " vertices, " << stats.levels << " levels" << std::endl;
+  std::cout << "embedded! in time " << timer[0] << "s" << std::endl;
+  for (size_t i = 0; i < coords.size(); i++)
+    for (int k = 0; k < dimension; k++)
+      if (std::isnan(coords[i][k])) {
+        std::cerr << "NaN at vertex " << vertices[i] << std::endl;
+        return 1;
+      }
+  return coords.size() == static_cast<size_t>(n) ? 0 : 2;
+}
+
 int main(int argc, char** argv) {
   std::string outdir;  // --out DIR: write the layout and the plot inputs like examples/embedder.cpp:230-289
-  bool coarsen = false, layout = false;
+  bool coarsen = false, layout = false, edges = false;
   for (int a = 1; a < argc; ++a) {
     if (a + 1 < argc && std::string(argv[a]) == "--gpus") return flat_on_gpus(std::atoi(argv[a + 1]), 2);
     if (a + 1 < argc && std::string(argv[a]) == "--out") outdir = argv[a + 1];
     if (std::string(argv[a]) == "--coarsen") coarsen = true;
     if (std::string(argv[a]) == "--layout") layout = true;
+    if (std::string(argv[a]) == "--edges") edges = true;
   }
   int nx = argc > 1 ? std::atoi(argv[1]) : 64, ny = nx;
   const int dimension = argc > 2 ? std::atoi(argv[2]) : 2;
   if (coarsen) return coarsen_then_embed(nx, dimension);
   if (layout) return layout_raw_graph(nx, dimension);
+  if (edges) return layout_edge_list(nx, dimension);
   std::vector<SparseMatrix> As = {grid(nx, ny)}, hierarchy;
   while (nx * ny > 40) {
     hierarchy.push_back(blocks(nx, ny));

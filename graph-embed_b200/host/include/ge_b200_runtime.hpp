@@ -2,6 +2,7 @@
 #ifndef GE_B200_RUNTIME_HPP
 #define GE_B200_RUNTIME_HPP
 
+#include <algorithm>
 #include <cstdlib>
 #include <stdexcept>
 #include <string>
@@ -175,6 +176,62 @@ inline std::vector<std::vector<double>> layout(const SparseMatrix& A, int d, dou
   std::vector<int> vert(n);
   int32_t k = 0;
   check(ge_layout_graph(default_context(), &a, d, 1, &copt, &eopt, x.data(), vert.data(), &k, stats));
+  vert.resize(static_cast<size_t>(k));
+  if (vertices) *vertices = vert;
+  x.resize(static_cast<size_t>(k) * d);
+  return unflatten(x, k, d);
+}
+
+// An edge list -> the SparseMatrix that linalgcpp's CooMatrix builds from it (ge_graph_from_edges):
+// Add(src[e], dst[e], w) for every edge, and Add(dst[e], src[e], w) too when symmetrising; duplicates
+// summed in that order; self-loops dropped unless edgeOptions->keep_self_loops.  weights null: 1.0;
+// edgeOptions null: symmetrise, drop self-loops, sum the weights.
+inline SparseMatrix fromEdges(int n, const std::vector<int>& src, const std::vector<int>& dst,
+                              const std::vector<double>* weights = nullptr,
+                              const ge_edges_options* edgeOptions = nullptr) {
+  if (src.size() != dst.size() || (weights && weights->size() != src.size()))
+    throw std::invalid_argument("graph-embed_b200: edge arrays differ in length");
+  const int64_t E = static_cast<int64_t>(src.size());
+  const bool sym = edgeOptions ? edgeOptions->symmetrize != 0 : true;
+  const size_t cap = static_cast<size_t>(std::max<int64_t>(E * (sym ? 2 : 1), 1));
+  std::vector<int> indptr(static_cast<size_t>(n) + 1), indices(cap);
+  std::vector<double> data(cap);
+  int64_t nnz = 0;
+  check(ge_graph_from_edges(default_context(), n, E, src.data(), dst.data(), weights ? weights->data() : nullptr,
+                            edgeOptions, indptr.data(), indices.data(), data.data(), static_cast<int64_t>(cap), &nnz,
+                            nullptr));
+  indices.resize(static_cast<size_t>(nnz));
+  data.resize(static_cast<size_t>(nnz));
+  return SparseMatrix(std::move(indptr), std::move(indices), std::move(data), n, n);
+}
+
+// ge_b200::layout from an edge list (ge_layout_edges): the graph fromEdges would return is built on
+// the device and laid out there without crossing PCIe.
+inline std::vector<std::vector<double>> layoutEdges(int n, const std::vector<int>& src, const std::vector<int>& dst,
+                                                    const std::vector<double>* weights, int d,
+                                                    double coarseningFactor, int minCoarse,
+                                                    std::vector<int>* vertices = nullptr,
+                                                    const ge_edges_options* edgeOptions = nullptr,
+                                                    ge_layout_stats* stats = nullptr) {
+  if (src.size() != dst.size() || (weights && weights->size() != src.size()))
+    throw std::invalid_argument("graph-embed_b200: edge arrays differ in length");
+  ge_coarsen_options copt;
+  ge_coarsen_options_default(&copt);
+  copt.coarsening_factor = coarseningFactor;
+  copt.min_coarse = minCoarse;
+  copt.seed = options().seed;
+  ge_embed_options eopt;
+  ge_embed_options_default(&eopt);
+  eopt.precision = options().precision;
+  eopt.seed = options().seed;
+  eopt.verbose = options().verbose;
+  const size_t nn = static_cast<size_t>(std::max(n, 0));
+  std::vector<double> x(nn * static_cast<size_t>(d));
+  std::vector<int> vert(nn);
+  int32_t k = 0;
+  check(ge_layout_edges(default_context(), n, static_cast<int64_t>(src.size()), src.data(), dst.data(),
+                        weights ? weights->data() : nullptr, edgeOptions, d, 1, &copt, &eopt, x.data(), vert.data(), &k,
+                        nullptr, stats));
   vert.resize(static_cast<size_t>(k));
   if (vertices) *vertices = vert;
   x.resize(static_cast<size_t>(k) * d);

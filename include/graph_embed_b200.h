@@ -290,6 +290,53 @@ ge_status ge_layout_graph(ge_context* ctx, const ge_csr* A, int dim, int32_t lar
                           double* coords_out, int32_t* vertices_out, int32_t* n_out,
                           ge_layout_stats* stats);
 
+/* ---- edge list -> graph on the device ------------------------------------------------------------ */
+/* The CSR that linalgcpp's CooMatrix (host/compat/sparsematrix.hpp) returns from ToSparse() after,
+ * for every edge e in order: skip it if src == dst and keep_self_loops == 0; Add(src, dst, w);
+ * then, if symmetrize and src != dst, Add(dst, src, w) (a kept self-loop is added once).  So the
+ * columns of each row are strictly ascending, duplicates are summed in that order starting from
+ * +0.0, and entries whose sum is zero are kept.  unit_weights = 1: every stored entry is 1.0 (with
+ * symmetrize = 1 and self-loops dropped, the canonical graph of graphs._finish). */
+typedef struct ge_edges_options {
+  int32_t symmetrize;      /* 1 */
+  int32_t keep_self_loops; /* 0 */
+  int32_t unit_weights;    /* 0 */
+} ge_edges_options;
+
+typedef struct ge_edges_stats {
+  double total_ms;            /* whole call */
+  double device_ms;           /* CUDA events from the first kernel to the end of the build */
+  int64_t nnz;                /* entries of the graph */
+  int64_t self_loops_dropped; /* edges skipped as self-loops */
+  int64_t duplicates_merged;  /* contributions added into an earlier one of the same entry */
+  int64_t kernel_launches;    /* one CUB sort counts as one launch */
+} ge_edges_stats;
+
+void ge_edges_options_default(ge_edges_options* opt);
+/* n vertices, E edges src[e] -> dst[e] (int32 ids in [0, n)) with weights w[e] (NULL: 1.0; when
+ * given, every weight must be finite, also with unit_weights).  opt NULL: defaults.  c_indptr:
+ * n + 1 entries, always filled, and *nnz_out always set; c_indices / c_data are filled when
+ * capacity >= *nnz_out -- capacity = 2E always suffices -- otherwise GE_ERR_INVALID is returned with
+ * *nnz_out set so the caller can retry.  GE_ERR_INVALID for an id outside [0, n), a non-finite
+ * weight, n < 0, E < 0, or more contributions than int32 row pointers can address (E > 2^30 - 1 when
+ * symmetrising, E > 2^31 - 1 otherwise).  On a multi-device context the call runs on the first
+ * device.  stats may be NULL. */
+ge_status ge_graph_from_edges(ge_context* ctx, int32_t n, int64_t E, const int32_t* src, const int32_t* dst,
+                              const double* w, const ge_edges_options* opt, int32_t* c_indptr,
+                              int32_t* c_indices, double* c_data, int64_t capacity, int64_t* nnz_out,
+                              ge_edges_stats* stats);
+/* Edge list -> coordinates: ge_graph_from_edges, then the body of ge_layout_graph on the graph it
+ * built, which stays on the device.  Only the edge arrays go up.  With eopt->seed != 0 the result
+ * (coordinates, vertices_out, n_out, status) equals ge_graph_from_edges followed by ge_layout_graph
+ * with the same options, bit for bit.  coords_out: n x dim capacity; vertices_out: n capacity (may
+ * be NULL).  edges_stats covers the graph build; layout_stats covers the whole call, the edge upload
+ * included.  Either may be NULL. */
+ge_status ge_layout_edges(ge_context* ctx, int32_t n, int64_t E, const int32_t* src, const int32_t* dst,
+                          const double* w, const ge_edges_options* edges_opt, int dim,
+                          int32_t largest_component, const ge_coarsen_options* copt,
+                          const ge_embed_options* eopt, double* coords_out, int32_t* vertices_out,
+                          int32_t* n_out, ge_edges_stats* edges_stats, ge_layout_stats* layout_stats);
+
 /* The reference's random stream: count draws of uniform_real_distribution<double>(-1,1) over
  * std::mt19937(seed) (include/forceatlas.hpp:104-108). */
 void ge_reference_uniform(uint32_t seed, int64_t count, double* out);
